@@ -2,12 +2,12 @@
 """Benchmark of the VAE-GAN training iteration (BASELINE.json metric: train images/s at 96x96,
 global batch 256, on 1/2/4/8 B200).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--global-batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--global-batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one full training iteration (G fwd, D(real), D(fake), D bwd + Adam, D(fake) again,
 G bwd + Adam) on one synthetic batch.  N > 1 is launched by torchrun (one rank per GPU, NCCL):
 the global batch is split over the ranks (strong scaling), BatchNorm statistics and gradients are
-all-reduced.  Prints ONE JSON line on rank 0.
+all-reduced.  Prints ONE JSON line on rank 0.  Every timed loop runs exactly K steps.
 
 `value`  : whole-job images/s with the batch already resident in HBM (CUDA-graph replay).
 `e2e`    : same metric through the public API with HOST batches: pinned H2D copy of every batch and a
@@ -213,7 +213,7 @@ def run_reference(args):
     og, od = O.OptState(), O.OptState()
     g = torch.Generator().manual_seed(1234)
     xs = [torch.rand(batch, 1, IMAGE, IMAGE, generator=g) for _ in range(2)]
-    steps = max(1, min(args.steps, 6))
+    steps = args.steps
     warm = max(1, min(args.warmup, 1))
     for i in range(warm):
         O.train_step(Pg, Pd, og, od, xs[i % 2], spec_g, spec_d)
@@ -343,6 +343,35 @@ def ncu_traffic(tag: str, batch: int):
     return None
 
 
+DUMP_MAX_ELEMS = 1 << 21        # 8 MB of float32 per array; the five large arrays stay well under 64 MB in all
+
+
+def dump_outputs(out_dir, losses, tr, G, D):
+    """--dump-outputs: what the last timed step handed its caller, one float32 DIR/<name>.npy per array - the step's
+    losses as read_losses() returns them (summed over the ranks), its reconstruction `gen`, latent `mu` / `log_var` and
+    discriminator logits `d_real` / `d_fake` / `d_gen` (NCHW order; with several GPUs these per-sample arrays are rank 0's
+    shard of the batch), and the trained networks as `G_state` / `D_state` (every floating-point state-dict entry,
+    flattened and concatenated in state-dict order).  An array of more than DUMP_MAX_ELEMS elements is stored as its
+    values at a fixed sample of flat indices (numpy default_rng(0), sorted), so two runs with the same arguments can be
+    compared element for element."""
+    import numpy as np
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    arrays = {k: torch.tensor(v, dtype=torch.float32) for k, v in losses.items()}
+    arrays.update(tr.last)
+    for tag, net in (("G", G), ("D", D)):
+        arrays[f"{tag}_state"] = torch.cat([v.detach().float().flatten() for v in net.state_dict().values()
+                                            if v.is_floating_point()])
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().float().contiguous().cpu().numpy()
+        if a.size > DUMP_MAX_ELEMS:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        np.save(out_dir / f"{name}.npy", a)
+        total += a.nbytes
+    assert total <= 64 << 20, f"--dump-outputs wrote {total} bytes"
+
+
 def run_decode_sweep(args):
     """BASELINE.json config 5: decoder-only sampling, z ~ N(0, I) of shape (B, 256, 24, 24) -> 96x96 image,
     eval mode (BatchNorm running statistics, no dropout), batch 1..4096 on one GPU, CUDA-graph replay.
@@ -418,7 +447,14 @@ def main():
     ap.add_argument("--optimizer", default="adam", choices=["adam", "rmsprop"])
     ap.add_argument("--workload", default="train", choices=["train", "cfg4", "decode"],
                     help="train: BASELINE metric (96x96, fs 64); cfg4: 256x256, widths x2; decode: config-5 sampling sweep")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (see dump_outputs); "
+                         "runs with deterministic (ordered) reductions so that runs with the same arguments match")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "decode"):
+        ap.error("--dump-outputs applies to the training step of --impl ours (--workload train or cfg4)")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -448,9 +484,14 @@ def main():
     assert args.global_batch % world == 0
     local_b = args.global_batch // world
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     peaks = measured_peaks()
     cdt = torch.float32 if args.fp32 else torch.bfloat16
+    if args.dump_outputs:
+        # outputs meant for comparison need ordered cross-block sums: with the default atomics the last bits of a step vary
+        # from run to run, and Adam's lr*sign(g) steps on near-zero gradients grow them into weights that differ by
+        # percents within a few dozen steps.  Without --dump-outputs the default (atomic) path is timed.
+        V.set_deterministic(True, dev)
 
     torch.manual_seed(0)
     with V.compute_dtype(cdt):
@@ -515,6 +556,8 @@ def main():
         ms_per_step = ms / K
         value = args.global_batch * K / (ms * 1e-3)
         losses = tr.read_losses()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, losses, tr, G, D)
 
         # ---------------- end to end: host batches in, losses out, every step ----------------
         # Public API: InputPipeline (pinned staging + copy stream, double buffered: the H2D copy of batch k+1 runs under
@@ -545,15 +588,14 @@ def main():
             pipe.get()                                                # drain the last prefetch
             return t
 
-        Ke = max(5, min(K, 20))
         pipe = V.InputPipeline(dev, (local_b, 1, IMAGE, IMAGE), torch.float32, normalize=False)
-        ms_e = e2e_run(pipe, host, Ke)
-        e2e_value = args.global_batch * Ke / (ms_e * 1e-3)
+        ms_e = e2e_run(pipe, host, K)
+        e2e_value = args.global_batch * K / (ms_e * 1e-3)
         # the same with RAW 8-bit pixels: 1 B/pixel over PCIe, per-image min-max normalisation on the device (SURVEY N3)
         host_u8 = [(h * 255.0).round().to(torch.uint8).pin_memory() for h in host]
         pipe8 = V.InputPipeline(dev, (local_b, 1, IMAGE, IMAGE), torch.uint8, normalize=True)
-        ms_e8 = e2e_run(pipe8, host_u8, Ke)
-        e2e_u8 = args.global_batch * Ke / (ms_e8 * 1e-3)
+        ms_e8 = e2e_run(pipe8, host_u8, K)
+        e2e_u8 = args.global_batch * K / (ms_e8 * 1e-3)
 
         roof = roof_hbm = cpu = lib = None
         # drop the captured graph (it holds NCCL work) on EVERY rank before any teardown
@@ -592,10 +634,10 @@ def main():
             },
             "clocks": clocks,
             "e2e": {"value": round(e2e_value, 2), "unit": "images/s", "h2d_bytes_per_step": local_b * IMAGE * IMAGE * 4 * world,
-                    "d2h_bytes_per_step": 7 * 4 * world, "steps": Ke, "ms_per_step": round(ms_e / Ke, 3),
+                    "d2h_bytes_per_step": 7 * 4 * world, "steps": K, "ms_per_step": round(ms_e / K, 3),
                     "api": "InputPipeline (pinned, copy stream, double buffered) -> VaeGanTrainer.step -> read_losses"},
             "e2e_u8_pipeline": {"value": round(e2e_u8, 2), "unit": "images/s", "h2d_bytes_per_step": local_b * IMAGE * IMAGE * world,
-                                "d2h_bytes_per_step": 7 * 4 * world, "steps": Ke, "ms_per_step": round(ms_e8 / Ke, 3),
+                                "d2h_bytes_per_step": 7 * 4 * world, "steps": K, "ms_per_step": round(ms_e8 / K, 3),
                                 "note": "raw uint8 pixels over PCIe, vg_normalize_images (per-image min-max, float64 math) on the copy stream"},
             "gpu_launches": int(launches_per_step * K),
             "launches_per_step": int(launches_per_step),
@@ -610,6 +652,8 @@ def main():
             "cpu_baseline": cpu,
             "losses_last_step": {k: round(v, 4) for k, v in losses.items()},
         }
+        if V.is_deterministic():
+            out["config"]["reductions"] = "deterministic (ordered cross-block sums)"
         print(json.dumps(out), flush=True)
     if world > 1:
         dist.barrier()

@@ -100,25 +100,45 @@ def test_blocks_every_mode(golden_dir):
                 check(P["b." + k].float(), v.float(), name + " " + k, rtol=1e-4, atol=1e-6)
 
 
-def test_reference_training_loop_two_iterations(golden_dir):
-    """The reference's own train_network_wgan (WGAN-GP + clamp + RMSprop) vs oracle.train_step."""
-    g = torch.load(golden_dir / "train_wgan_gp_2iters.pt")
-    spec_g = O.GeneratorSpec(**g["spec_g"])
-    spec_d = O.DiscriminatorSpec(**g["spec_d"])
+def _reference_loop_oracle(g, spec_g, spec_d):
+    """oracle.train_step twice on the stored inputs (WGAN-GP + clamp + RMSprop); returns (Pg, Pd, per-iteration losses)."""
     Pg = O.make_generator_params(spec_g, seed=g["seed_g"])
     Pd = O.make_discriminator_params(spec_d, seed=g["seed_d"])
     og = O.OptState(kind="rmsprop", lr=3e-4, weight_decay=1e-5)
     od = O.OptState(kind="rmsprop", lr=3e-4, weight_decay=1e-5)
+    outs = []
+    for i in range(2):
+        dm = g["d_masks"][i]
+        outs.append(O.train_step(Pg, Pd, og, od, g["xs"][i].float(), spec_g, spec_d,
+                                 eps_noise=g["epss"][i], g_masks=g["g_masks"][i], d_masks_real=dm[0],
+                                 d_masks_fake=dm[1], d_masks_gp=dm[2], d_masks_gen=dm[3],
+                                 loss_mode="wgan_gp", gp_alpha=g["alphas"][i]))
+    return Pg, Pd, outs
+
+
+def test_reference_training_loop_two_iterations(golden_dir):
+    """The reference's own train_network_wgan (WGAN-GP + clamp + RMSprop) vs oracle.train_step.
+
+    A few hundred of the ~146k stored parameter / buffer elements have no machine-independent fp32 value: their gradients
+    are zero in exact arithmetic (e.g. the bias of a BatchNorm that only feeds other BatchNorms), RMSprop's first steps
+    scale that rounding noise to a full step, and the BatchNorm statistics and spectral-norm vectors downstream follow.
+    The CPU's summation order (thread count, vector kernels) decides them, so the oracle is also run at other thread
+    counts here, and each element may deviate from the reference by the spread those runs show on it, times NOISE_SLACK
+    (four runs on one machine under-cover another CPU's result by up to ~6x, measured with AVX2 kernels against the
+    AVX-512 golden).  Every element the oracle reproduces across summation orders keeps the plain tolerance.
+    The thread-count spread measured on one kind of kernel does not bound every other kind: with torch's scalar CPU
+    kernels (ATEN_CPU_CAPABILITY=default) one running_mean element still lands outside it, so on a CPU without AVX2 or
+    AVX-512 kernels (e.g. some aarch64 hosts) this test can fail without any change to the oracle."""
+    NOISE_SLACK = 8.0
+    g = torch.load(golden_dir / "train_wgan_gp_2iters.pt")
+    spec_g = O.GeneratorSpec(**g["spec_g"])
+    spec_d = O.DiscriminatorSpec(**g["spec_d"])
+    Pg, Pd, outs = _reference_loop_oracle(g, spec_g, spec_d)
     logged = re.findall(r"\[D loss: ([-\d.e+]+)\] \[G loss: ([-\d.e+]+)\] \[Recon loss: ([-\d.e+]+)\] \[KL: ([-\d.e+]+)\]",
                         g["log"])
     assert len(logged) == 2
-    for i in range(2):
-        dm = g["d_masks"][i]
-        out = O.train_step(Pg, Pd, og, od, g["xs"][i].float(), spec_g, spec_d,
-                           eps_noise=g["epss"][i], g_masks=g["g_masks"][i], d_masks_real=dm[0],
-                           d_masks_fake=dm[1], d_masks_gp=dm[2], d_masks_gen=dm[3],
-                           loss_mode="wgan_gp", gp_alpha=g["alphas"][i])
-        d_l, g_l, r_l, k_l = (float(v) for v in logged[i])
+    for out, logged_i in zip(outs, logged):
+        d_l, g_l, r_l, k_l = (float(v) for v in logged_i)
         assert abs(float(out["d_loss"]) - d_l) <= 2e-3 + 1e-3 * abs(d_l)
         assert abs(float(out["g_loss"]) - g_l) <= 2e-3 + 1e-4 * abs(g_l)
         assert abs(float(out["recon"]) - r_l) <= 2e-3
@@ -126,10 +146,32 @@ def test_reference_training_loop_two_iterations(golden_dir):
     # known-answer from the notebook's own log (README.md:971-972): after the first clamp
     # the critic loss sits at ~lambda_gp * 1
     assert abs(float(out["d_loss"]) - 10.0) < 0.05
-    for k, v in g["g_after"].items():
-        check(Pg[k].float(), v if not isinstance(v, torch.Tensor) else v.float(), "G." + k, rtol=2e-4, atol=1e-5)
-    for k, v in g["d_after"].items():
-        check(Pd[k].float(), v if not isinstance(v, torch.Tensor) else v.float(), "D." + k, rtol=2e-4, atol=1e-5)
+    threads = torch.get_num_threads()
+    try:
+        others = []
+        for n in (1, 3, 16):
+            torch.set_num_threads(n)
+            others.append(_reference_loop_oracle(g, spec_g, spec_d)[:2])
+    finally:
+        torch.set_num_threads(threads)
+    for tag, i, after in (("G", 0, g["g_after"]), ("D", 1, g["d_after"])):
+        P = (Pg, Pd)[i]
+        for k, v in after.items():
+            if not isinstance(v, torch.Tensor) and not (isinstance(v, dict) and v.get("summary")):
+                check(P[k].float(), v, f"{tag}.{k}", rtol=2e-4, atol=1e-5)
+                continue
+            runs = torch.stack([Q[i][k].detach().float().flatten() for Q in others] + [P[k].detach().float().flatten()])
+            got = runs[-1]
+            spread = runs.amax(0) - runs.amin(0)
+            if isinstance(v, dict):
+                got, spread, want = got[:: v["stride"]][:4096], spread[:: v["stride"]][:4096], v["sample"].float()
+                assert abs(float(runs[-1].double().abs().sum()) - v["asum"]) <= 1e-4 * max(1.0, v["asum"]), f"{tag}.{k}"
+            else:
+                want = v.float().flatten()
+            excess = (got - want).abs() - (1e-5 + 2e-4 * want.abs() + NOISE_SLACK * spread)
+            assert float(excess.max()) <= 0.0, \
+                f"{tag}.{k}: {int((excess > 0).sum())} of {want.numel()} elements off the reference by up to " \
+                f"{float((got - want).abs().max()):.3e} beyond tolerance + {NOISE_SLACK} x summation-order spread"
 
 
 def test_structure_matches_reference_state_dict(golden_dir):
