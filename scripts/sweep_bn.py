@@ -1,5 +1,5 @@
 """Time the BatchNorm-family kernels on the 128-channel 96x96 tensor (batch 64 = 151 MB) with CUDA events."""
-import ctypes as C, os, sys
+import ctypes as C, sys
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
 import torch
@@ -33,7 +33,7 @@ cases = {
   "bwd_apply (3x)": (3, lambda: _lib.call("vg_bn_act_backward_apply", dy.data_ptr(), x.data_ptr(), mr.data_ptr(), gamma.data_ptr(), beta.data_ptr(), sums.data_ptr(), float(B*H*H), C.byref(d), None, None, dx.data_ptr(), s)),
   "bn_add+stats (3x)": (3, lambda: _lib.call("vg_bn_add_forward", x.data_ptr(), None, None, None, dy.data_ptr(), mr.data_ptr(), gamma.data_ptr(), beta.data_ptr(), C.byref(d), y.data_ptr(), sums.data_ptr(), s)),
 }
-print(f"C={Cc} tensor {MB:.0f} MB  REDUCE_BPS={os.environ.get('VG_BN_REDUCE_BPS','3')} APPLY_BPS={os.environ.get('VG_BN_APPLY_BPS','8')}")
+print(f"C={Cc} tensor {MB:.0f} MB")
 for name, (mult, fn) in cases.items():
     t = timeit(fn)
     print(f"  {name:20s} {t*1e3:7.1f} us  {mult*MB/t/1e3:6.2f} TB/s  {100*mult*MB/t/1e3/6.5389:5.1f}% of measured HBM")

@@ -1,7 +1,6 @@
 """Time every tensor-core layer shape of the step (fwd / dgrad / wgrad) with CUDA events.
-usage: python scripts/sweep_conv.py [batch]      (env VG_TC_BN=64|128|256 forces the N tile)"""
+usage: python scripts/sweep_conv.py [batch]"""
 import ctypes as C
-import os
 import sys
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
@@ -38,7 +37,7 @@ def timeit(fn, iters=8):
     ts = sorted(a.elapsed_time(b) for a, b in evs)
     return sum(ts[1:-1]) / (len(ts) - 2)
 
-print(f"batch {B}  VG_TC_BN={os.environ.get('VG_TC_BN', 'auto')}")
+print(f"batch {B}")
 tot = {"fwd": 0.0, "fwd+stats": 0.0, "dgrad": 0.0, "wgrad": 0.0}
 for name, cin, cout, h, k, st, pad, tr in SHAPES:
     geom = VF.ConvGeom(k, st, pad, tr)

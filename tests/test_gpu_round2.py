@@ -156,8 +156,8 @@ def test_bn_stream_add_forward_backward(dtype, shape, bn_a, bn_b, slope):
 
 
 def test_bn_stream_matches_register_kernels_bitwise_on_statistics():
-    """The streaming statistics kernel and the register-staged one (VG_BN_STREAM=0 path, still used for odd channel
-    counts) accumulate the same fp32 partial sums only approximately - but both must agree with an fp64 reduction
+    """The streaming statistics kernel and the register-staged one (used for odd channel counts and unaligned
+    tensors) accumulate the same fp32 partial sums only approximately - but both must agree with an fp64 reduction
     to 1e-6 relative on a 75 MB tensor."""
     vf = VF()
     from vae_gan_b200 import _lib

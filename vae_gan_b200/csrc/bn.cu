@@ -48,17 +48,8 @@ static inline int grid_for(long long rows, int rpb, int iters_target = kUnroll *
 // kernels that end in a per-channel reduction: every block issues 2C same-address fp64 atomics, which
 // serialise in L2 - keep the block count at a small multiple of the SM count and give each block
 // more rows instead.
-static int reduce_blocks_per_sm() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VG_BN_REDUCE_BPS"); v = e ? atoi(e) : 3; if (v < 1) v = 1; }
-  return v;
-}
-static int apply_blocks_per_sm() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VG_BN_APPLY_BPS"); v = e ? atoi(e) : 4; if (v < 1) v = 1; }
-  return v;
-}
-#define kReduceBlocksPerSm reduce_blocks_per_sm()
+constexpr int kReduceBlocksPerSm = 3;
+constexpr int kApplyBlocksPerSm = 4;
 
 // 16-bit Philox keep decisions for 8 consecutive elements starting at linear index e0 (e0 % 8 == 0)
 __device__ __forceinline__ void keep8(const Philox& ph, unsigned long long e0, uint32_t thr16, bool keep[8]) {
@@ -937,7 +928,7 @@ static int bn_act_backward_t(const T* dy, const T* x, const float* mr, const flo
     long long rows = k.fold ? d->rows / 8 : d->rows;
     k.rows = rows;
     RowMap m = make_rowmap(k.fold ? 8 : d->c);
-    int grid = grid_for(rows, m.rpb, APPLY ? kUnroll : kUnrollWide, APPLY ? apply_blocks_per_sm() : kReduceBlocksPerSm);
+    int grid = grid_for(rows, m.rpb, APPLY ? kUnroll : kUnrollWide, APPLY ? kApplyBlocksPerSm : kReduceBlocksPerSm);
     size_t sm = APPLY ? 0 : vec_smem();
     double* part = nullptr;
     if (!APPLY && g_det.on && !(part = (double*)det_scratch((size_t)grid * 2 * d->c * sizeof(double)))) return VG_EINVAL;
@@ -1020,7 +1011,7 @@ static int bn_dbl_bwd_t(const T* dy, const T* x, const T* G, const float* mean_r
                         T* g_x, cudaStream_t s) {
   BnK k = make_bnk(d);
   RowMap m = make_rowmap(d->c);
-  int grid = grid_for(d->rows, m.rpb, kUnroll, APPLY ? apply_blocks_per_sm() : kReduceBlocksPerSm);
+  int grid = grid_for(d->rows, m.rpb, kUnroll, APPLY ? kApplyBlocksPerSm : kReduceBlocksPerSm);
   const size_t smem = APPLY ? 0 : (size_t)5 * 8 * kBnThreads * sizeof(float);
   double* part = nullptr;
   if (!APPLY && g_det.on && !(part = (double*)det_scratch((size_t)grid * 5 * d->c * sizeof(double)))) return VG_EINVAL;
@@ -1076,7 +1067,7 @@ static int bn_add_t(const T* a, const float* mra, const float* ga, const float* 
     long long rows = k.fold ? d->rows / 8 : d->rows;
     k.rows = rows;
     RowMap m = make_rowmap(k.fold ? 8 : d->c);
-    int grid = grid_for(rows, m.rpb, kUnroll, stats ? kReduceBlocksPerSm : apply_blocks_per_sm());
+    int grid = grid_for(rows, m.rpb, kUnroll, stats ? kReduceBlocksPerSm : kApplyBlocksPerSm);
     double* part = nullptr;
     if (stats && g_det.on && !(part = (double*)det_scratch((size_t)grid * 2 * d->c * sizeof(double)))) return VG_EINVAL;
     if (stats)

@@ -59,7 +59,11 @@ struct Args {
   int cg;                // channel groups per row (c / 8; 1 when folded)
   int tpb;               // consumer threads in use = (256 / cg) * cg
   int fold;              // single-channel tensor viewed as [rows / 8][8]
-  int reverse;           // walk the tiles from the END of the tensor (see bn_stream_reverse())
+  // L2 reuse between consecutive passes over the same tensor: a producer (convolution, previous pass) leaves the END of
+  // the tensor it wrote / read last in the 126 MB L2.  The reduction-type passes (statistics, backward reduce, residual
+  // add) therefore walk the tensor backwards (reverse = 1) - they start on the freshest lines - and the apply passes that
+  // follow them walk forwards, starting on what the reduction touched last.
+  int reverse;
   int hw;
   Chan A, B;
   // reductions
@@ -422,11 +426,7 @@ __global__ void __launch_bounds__(kThreads, 2) bn_stream_kernel(const __grid_con
 // ------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------
-static int ctas_per_sm() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VG_BN_STREAM_CTAS"); v = e ? atoi(e) : 2; if (v < 1) v = 1; }
-  return v;
-}
+constexpr int kCtasPerSm = 2;
 
 // folded (single-channel) tensors in deterministic mode: partials[block][q][warp] -> sums_out[q * c] (c == 1), one thread
 // per quantity walking blocks and warps in order (a few thousand fp64 adds)
@@ -455,7 +455,7 @@ static int launch(const Args& a, cudaStream_t s) {
     attr_err = cudaFuncSetAttribute(bn_stream_kernel<T, MODE, DROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, G::kSmemBytes);
   });
   VG_CUDA(attr_err);
-  const long long cap = (long long)num_sms() * ctas_per_sm();
+  const long long cap = (long long)num_sms() * kCtasPerSm;
   const int grid = (int)std::max<long long>(1, std::min<long long>(a.ntiles, cap));
   if (ModeTraits<MODE>::kReduce && g_det.on) {
     // deterministic mode: per-block partial sums, added in block order by a second tiny kernel.  A folded single-channel
@@ -484,26 +484,10 @@ static int launch_drop(const Args& a, cudaStream_t s) {
 
 }  // namespace bs
 
-// L2 reuse between consecutive passes over the same tensor: a producer (convolution, previous pass) leaves the END of
-// the tensor it wrote / read last in the 126 MB L2.  The reduction-type passes (statistics, backward reduce, residual
-// add) therefore walk the tensor backwards - they start on the freshest lines - and the apply passes that follow them
-// walk forwards, starting on what the reduction touched last.  VG_BN_REVERSE=0 disables it (A/B).
-static bool bn_stream_reverse() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VG_BN_REVERSE"); v = e ? atoi(e) : 1; }
-  return v != 0;
-}
-
-bool bn_stream_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("VG_BN_STREAM"); v = e ? atoi(e) : 1; }
-  return v != 0;
-}
-
 // can the streaming kernels take this tensor?  (vector path: C % 8 == 0 and C / 8 <= 256; folded path: C == 1 and
 // rows % 8 == 0; every streamed pointer 16-byte aligned)
 bool bn_stream_ok(const VgBnDesc* d, const void* p0, const void* p1, const void* p2, const void* p3) {
-  if (!bn_stream_enabled() || d->rows <= 0) return false;
+  if (d->rows <= 0) return false;
   const bool vec = d->c % 8 == 0 && d->c / 8 <= bs::kConsumers;
   const bool fold = d->c == 1 && d->rows % 8 == 0;
   if (!vec && !fold) return false;
@@ -577,7 +561,7 @@ int bn_stream_stats(const void* x, const VgBnDesc* d, double* sums, cudaStream_t
   a.in0 = x;
   a.sums_out = sums;
   a.thr16 = 0;
-  a.reverse = bn_stream_reverse();
+  a.reverse = 1;
   return dispatch<bs::kStats>(a, d, s);
 }
 
@@ -601,7 +585,7 @@ int bn_stream_bwd_reduce(const void* dy, const void* x, const float* mean_rstd, 
   a.A.gamma = gamma;
   a.A.beta = beta;
   a.sums_out = sums;
-  a.reverse = bn_stream_reverse();
+  a.reverse = 1;
   return dispatch<bs::kBwdReduce>(a, d, s);
 }
 
@@ -654,7 +638,7 @@ int bn_stream_add(const void* x0, const VgBnChannel* bn_a, const void* x1, const
   set_chan(a.B, bn_b, d->training);
   a.sums_out = stats;
   a.thr16 = 0;
-  a.reverse = bn_stream_reverse();
+  a.reverse = 1;
   if (stats != nullptr) return dispatch<bs::kAddStats>(a, d, s);
   return dispatch<bs::kAdd>(a, d, s);
 }

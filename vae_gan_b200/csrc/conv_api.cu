@@ -14,8 +14,7 @@ int simt_pack_weights_batched(const VgPackItem* items, int n_items, int dtype, c
 bool tc_conv_supported(const VgConvDesc*, bool dgrad);
 bool tc_wgrad_supported(const VgConvDesc*);
 int tc_conv_run(const VgConvDesc*, bool dgrad, const void* in, const void* wpack, const float* bias, const float* colscale,
-                const float* sigma, int sigma_group_n, void* out, int out_dtype, double* stats, bool* stats_fused, cudaStream_t,
-                const VgConvEpilogue* ep = nullptr);
+                const float* sigma, int sigma_group_n, void* out, int out_dtype, cudaStream_t, const VgConvEpilogue* ep = nullptr);
 int tc_wgrad_run(const VgConvDesc*, const void* x, const void* dy, float* dw, float* workspace, cudaStream_t, bool acc_only = false);
 int sn_backward_run(const float* dw_hat, const float* w_orig, const float* u, const float* v, const float* sigma, int rows, int cols,
                     float* dw_orig, float* dot_ws, cudaStream_t s);
@@ -90,16 +89,21 @@ extern "C" int vg_conv_forward_fused(const VgConvDesc* d, const void* x, const v
   const int sigma_group_n = ep->sigma_group_n;
   const bool inference_ep = ep->act_slope != 1.0f || ep->residual != nullptr || ep->y2 != nullptr;
   cudaStream_t s = as_stream(stream);
-  bool stats_fused = false;
   if (tc_conv_supported(d, false) && !(d->c_out == 1 && colscale != nullptr))
-    rc = tc_conv_run(d, false, x, pack_kn, bias, colscale, sigma, sigma_group_n, y, d->out_dtype, stats, &stats_fused, s, ep);
+    rc = tc_conv_run(d, false, x, pack_kn, bias, colscale, sigma, sigma_group_n, y, d->out_dtype, s, ep);
   else if (inference_ep) {
     set_error("the activation / residual / second-output epilogue exists on the tensor-core path only (bf16, channels %% 64 == 0)");
     return VG_EUNSUPPORTED;
   } else
     rc = simt_conv_forward(d, x, pack_nk, bias, colscale, sigma, sigma_group_n, y, s);
   if (rc) return rc;
-  if (stats != nullptr && !stats_fused) {
+  // BatchNorm statistics of y come from the separate streaming statistics kernel.  Accumulating them in the tensor-core
+  // epilogue was measured slower on B200 twice and removed: with per-chunk shared-memory transposes +35 % per launch (8
+  // epilogue warps) / +60 % (4) against a 20 us statistics kernel; with a 31-shuffle column sum per 32 x 32 chunk in every
+  // kernel form (scripts/sweep_conv.py, batch 64) 64->64 @96 74.9 -> 163 us, 128->128 @96 151 -> 217 us, 512->512 @24
+  // 110 -> 125 us, whole step 63.7 -> 68.2 ms against a 17 us kernel: the epilogue warps bound the short-reduction layers
+  // and ~350 extra instructions per chunk double their work.
+  if (stats != nullptr) {
     VgBnDesc b{};
     b.rows = (long long)d->n * d->h_out * d->w_out;
     b.c = d->c_out;
@@ -125,7 +129,7 @@ extern "C" int vg_conv_dgrad_scaled(const VgConvDesc* d, const void* dy, const v
   VG_CHECK_ARG(sigma_group_n >= 0, "sigma_group_n must be >= 0");
   cudaStream_t s = as_stream(stream);
   if (tc_conv_supported(d, true))
-    return tc_conv_run(d, true, dy, pack_nk, nullptr, nullptr, sigma, sigma_group_n, dx, d->act_dtype, nullptr, nullptr, s);
+    return tc_conv_run(d, true, dy, pack_nk, nullptr, nullptr, sigma, sigma_group_n, dx, d->act_dtype, s);
   return simt_conv_dgrad(d, dy, pack_kn, sigma, sigma_group_n, dx, s);
 }
 

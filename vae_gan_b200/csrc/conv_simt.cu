@@ -790,9 +790,7 @@ __global__ void __launch_bounds__(degs::kThreads, 1) wgrad_degenerate_stream_ker
 template <typename T>
 static int try_degenerate_stream(bool flip, const void* V, const void* S, int n, int h, int w, int c, float* dw, cudaStream_t s, bool* taken) {
   *taken = false;
-  static int on = -1;
-  if (on < 0) { const char* e = getenv("VG_DEG_STREAM"); on = e ? atoi(e) : 1; }
-  if (!on || g_det.on) return VG_OK;      // deterministic mode: the strip kernel has the ordered reduction
+  if (g_det.on) return VG_OK;      // deterministic mode: the strip kernel has the ordered reduction
   const int groups = c / 8;
   if (c % 8 != 0 || groups > 256 || 256 % groups != 0 || w % 8 != 0) return VG_OK;
   if (((size_t)w * sizeof(T)) % 16 != 0 || ((uintptr_t)V & 15) != 0 || ((uintptr_t)S & 15) != 0) return VG_OK;

@@ -61,7 +61,6 @@ struct alignas(64) TcConvParams {
   const float* colscale;
   const float* sigma;    // nullable: the accumulator is multiplied by 1 / sigma[group] (spectral norm applied in the epilogue,
   int sigma_group_n;     //   so the packed weights stay valid across forwards); group = sample / sigma_group_n (0: one group)
-  double* stats;         // nullable: [2*n_out] per-channel sum / sum of squares of the stored output
   // inference epilogue (BatchNorm-folded sampling path, bf16 outputs only; see VgConvEpilogue in the header)
   float act_slope;       // LeakyReLU slope of the stored output (1 = none)
   const void* residual;  // nullable: same shape/dtype as out, added (after rounding the accumulator to bf16) before the activation
@@ -94,39 +93,14 @@ constexpr int kTcThreads = 256;
 constexpr int kABytes = 128 * 128;   // 128 rows x 64 bf16
 constexpr int kStageBytes = 32 * 64;  // per epilogue warp: 32 rows x 32 bf16 of one output chunk (coalescing transpose)
 
-template <int BN, int MT, int STAGES>
+template <int BN, int STAGES>
 struct ConvSmem {
   static constexpr int kBBytes = BN * 128;
-  static constexpr int kBytes = STAGES * (MT * kABytes + kBBytes) + (2 * STAGES + 1) * 8 + 16 + 1024 + 4 * kStageBytes + 16 + 512;
+  static constexpr int kBytes = STAGES * (kABytes + kBBytes) + (2 * STAGES + 1) * 8 + 16 + 1024 + 4 * kStageBytes + 16 + 512;
 };
 
-
-// Column sums of a 32 x 32 block held one ROW per lane (v[j] = column j): recursive halving over the lane bits - in step H
-// the lanes with bit H set keep the upper H columns of what they hold and receive the lower lanes' share of them (and vice
-// versa), so after the steps 16, 8, 4, 2, 1 lane l holds the sum of column l over all 32 rows.  31 shuffles, all register
-// indices static.  (Round 1 transposed through shared memory instead: 1.5 k shared accesses per chunk, measured +35..60 %.)
-template <int H>
-__device__ __forceinline__ void fold_cols(float (&v)[32], bool up) {
-#pragma unroll
-  for (int k = 0; k < H; ++k) {
-    const float send = up ? v[k] : v[k + H];
-    const float keep = up ? v[k + H] : v[k];
-    v[k] = keep + __shfl_xor_sync(0xffffffffu, send, H);
-  }
-}
-__device__ __forceinline__ float colsum32(float (&v)[32], int lane) {
-  fold_cols<16>(v, (lane & 16) != 0);
-  fold_cols<8>(v, (lane & 8) != 0);
-  fold_cols<4>(v, (lane & 4) != 0);
-  fold_cols<2>(v, (lane & 2) != 0);
-  fold_cols<1>(v, (lane & 1) != 0);
-  return v[0];
-}
-
 // Finishes one 32-column chunk of one accumulator row per thread: 1/sigma, bias, Dropout2d column scale, store
-// (bf16 / fp32 / split-K vector reductions / single channel) and - with `do_stats` - adds this warp's per-column sum
-// and sum of squares of the values AS STORED to (st_sum, st_sq): lane l owns column l.  Those feed the BatchNorm
-// that follows the convolution (README.md:192), saving a full read of y by a separate statistics kernel.
+// (bf16 / fp32 / split-K vector reductions / single channel).
 //
 // bf16 outputs go through `stage` (a 2 KB per-warp shared-memory buffer) when it is given: lane = pixel row holds 64 B of
 // consecutive channels, so a direct 16-byte store per lane touches 32 different 128-byte lines per instruction - the
@@ -135,9 +109,9 @@ __device__ __forceinline__ float colsum32(float (&v)[32], int lane) {
 // reads it back transposed and stores with FOUR consecutive lanes covering one row's 64 bytes: 8 lines per instruction.
 template <bool INF>
 __device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint32_t (&r)[32], bool valid, bool add_bias,
-                                               long long opix, int gn, int ncol, bool first_chunk, bool do_stats, int lane,
-                                               float& st_sum, float& st_sq, uint8_t* stage = nullptr, int sx = 0, int sy = 0,
-                                               int sn = 0, int out_phase = 0) {
+                                               long long opix, int gn, int ncol, bool first_chunk, uint8_t* stage = nullptr,
+                                               int sx = 0, int sy = 0, int sn = 0, int out_phase = 0) {
+  const int lane = threadIdx.x & 31;
   float v[32];
 #pragma unroll
   for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -290,34 +264,20 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint
       }
     }
   }
-  if (do_stats) {
-    float q[32];
-#pragma unroll
-    for (int j = 0; j < 32; ++j) {
-      const float a = valid ? (p.out_f32 ? v[j] : __bfloat162float(__float2bfloat16_rn(v[j]))) : 0.f;
-      v[j] = a;
-      q[j] = a * a;
-    }
-    st_sq += colsum32(q, lane);
-    st_sum += colsum32(v, lane);
-  }
 }
 
 // ------------------------------------------------------------------------------------------
 // forward / dgrad implicit GEMM
 // ------------------------------------------------------------------------------------------
-// MT pixel tiles (128 rows each) per CTA share every weight tile: B traffic per FLOP drops by MT
-// (the implicit GEMM re-reads its operands from L2 for every tap, so it is L2-bandwidth bound
-// unless each staged byte feeds enough MMAs).
-template <int BN, int MT, int STAGES, bool INF>
+// one-shot form: one CTA per (128-pixel tile, N tile, phase | k-split)
+template <int BN, int STAGES, bool INF>
 __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_constant__ TcConvParams p) {
   extern __shared__ uint8_t smem_raw[];
   constexpr int kBBytes = BN * 128;
-  constexpr int kAStage = MT * kABytes;
   const uint32_t raw_addr = ptx::smem_u32(smem_raw);
   uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
   uint8_t* sA = smem;
-  uint8_t* sB = smem + STAGES * kAStage;
+  uint8_t* sB = smem + STAGES * kABytes;
   uint64_t* full = reinterpret_cast<uint64_t*>(sB + STAGES * kBBytes);
   uint64_t* empty = full + STAGES;
   uint64_t* tmem_full = empty + STAGES;
@@ -331,17 +291,13 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
   const int kb0 = p.ksplit > 1 ? (int)blockIdx.z * p.k_per_split : 0;
   const int kb1 = p.ksplit > 1 ? min(ntaps * p.k_chunks, kb0 + p.k_per_split) : ntaps * p.k_chunks;
   const int num_k = max(0, kb1 - kb0);
-  const int total_tiles = p.tiles_x * p.tiles_y * p.tiles_n;
-  const int tile0 = blockIdx.x * MT;
-  const int nvalid = min(MT, total_tiles - tile0);
-  int x0s[MT], y0s[MT], n0s[MT];
-#pragma unroll
-  for (int i = 0; i < MT; ++i) {
-    int t = min(tile0 + i, total_tiles - 1);
+  int x0, y0, n0;
+  {
+    int t = blockIdx.x;
     const int tx = t % p.tiles_x; t /= p.tiles_x;
     const int ty = t % p.tiles_y;
     const int tn = t / p.tiles_y;
-    x0s[i] = tx * p.TW; y0s[i] = ty * p.TH; n0s[i] = tn * p.TN;
+    x0 = tx * p.TW; y0 = ty * p.TH; n0 = tn * p.TN;
   }
   const int ncol0 = blockIdx.y * BN;
 
@@ -357,8 +313,7 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
     ptx::mbar_init(tmem_full, 1);
     ptx::fence_barrier_init();
   }
-  constexpr int kTmemCols = (MT * BN < 32) ? 32 : MT * BN;
-  if (warp == 2) ptx::tmem_alloc<kTmemCols>(tmem_slot);
+  if (warp == 2) ptx::tmem_alloc<BN>(tmem_slot);
   ptx::tc_fence_before();
   __syncthreads();
   ptx::tc_fence_after();
@@ -377,11 +332,8 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
         const CUtensorMap* im = &p.in_maps[tap.map];
         ptx::mbar_wait(&empty[stage], phase ^ 1u);
         if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(&full[stage], nvalid * kABytes + kBBytes);
-#pragma unroll
-          for (int m = 0; m < MT; ++m)
-            if (m < nvalid)
-              ptx::tma_load_4d(sA + stage * kAStage + m * kABytes, im, &full[stage], kc * 64, x0s[m] + tap.dx, y0s[m] + tap.dy, n0s[m]);
+          ptx::mbar_arrive_expect_tx(&full[stage], kABytes + kBBytes);
+          ptx::tma_load_4d(sA + stage * kABytes, im, &full[stage], kc * 64, x0 + tap.dx, y0 + tap.dy, n0);
           ptx::tma_load_2d(sB + stage * kBBytes, &p.w_map, &full[stage], kc * 64, tap.wrow + ncol0);
         }
         __syncwarp();
@@ -400,19 +352,14 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
         ptx::tc_fence_after();
         if (ptx::elect_one()) {
 #pragma unroll
-          for (int m = 0; m < MT; ++m) {
-            if (m < nvalid) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                ptx::mma_bf16_ss_lohi(tmem_base + (uint32_t)(m * BN), a_lo + (uint32_t)((m * kABytes + k * 32) >> 4),
-                                      b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc, (i | k) != 0);
-            }
-          }
+          for (int k = 0; k < 4; ++k)
+            ptx::mma_bf16_ss_lohi(tmem_base, a_lo + (uint32_t)((k * 32) >> 4), b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc,
+                                  (i | k) != 0);
           ptx::mma_commit(&empty[stage]);
         }
         __syncwarp();
         if (++stage == STAGES) { stage = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
-        else { a_lo += (uint32_t)(kAStage >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
+        else { a_lo += (uint32_t)(kABytes >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
       }
       if (ptx::elect_one()) ptx::mma_commit(tmem_full);
       __syncwarp();
@@ -433,45 +380,28 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
       ptx::mbar_wait(tmem_full, 0);
       ptx::tc_fence_after();
     }
-    const bool do_stats = p.stats != nullptr && p.ksplit <= 1 && num_k > 0;
-    float st_s[BN / 32], st_q[BN / 32];
-#pragma unroll
-    for (int c = 0; c < BN / 32; ++c) st_s[c] = st_q[c] = 0.f;
     // deterministic split-K: this split's reductions go after those of split z - 1 of the same output tile
     int* const det_lock = (p.det_locks != nullptr && p.ksplit > 1) ? p.det_locks + (blockIdx.y * gridDim.x + blockIdx.x) : nullptr;
     if (det_lock) {
       if (lane == 0) det_wait_turn(det_lock, (int)blockIdx.z);
       __syncwarp();
     }
-#pragma unroll 1
-    for (int m = 0; m < nvalid; ++m) {
-      const int gx = x0s[m] + xl, gy = y0s[m] + yl, gn = n0s[m] + nl;
-      const bool valid = gx < p.gw && gy < p.gh && gn < p.gn && !(p.ksplit > 1 && num_k == 0 && p.det_split_stride == 0);
-      const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
+    const int gx = x0 + xl, gy = y0 + yl, gn = n0 + nl;
+    const bool valid = gx < p.gw && gy < p.gh && gn < p.gn && !(p.ksplit > 1 && num_k == 0 && p.det_split_stride == 0);
+    const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
 #pragma unroll
-      for (int c = 0; c < BN / 32; ++c) {
-        const int c0 = c * 32;
-        uint32_t r[32];
-        if (num_k > 0) {
-          ptx::tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(m * BN + c0), r);
-          ptx::tmem_ld_wait();
-        } else {
+    for (int c = 0; c < BN / 32; ++c) {
+      const int c0 = c * 32;
+      uint32_t r[32];
+      if (num_k > 0) {
+        ptx::tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
+        ptx::tmem_ld_wait();
+      } else {
 #pragma unroll
-          for (int j = 0; j < 32; ++j) r[j] = 0u;
-        }
-        epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || blockIdx.z == 0, opix, gn, ncol0 + c0, c == 0, do_stats, lane, st_s[c], st_q[c],
-                       stage_base + q * kStageBytes, x0s[m] + xl0, y0s[m] + yl0, n0s[m] + nl0, (int)blockIdx.z);
+        for (int j = 0; j < 32; ++j) r[j] = 0u;
       }
-    }
-    if (do_stats) {
-#pragma unroll
-      for (int c = 0; c < BN / 32; ++c) {
-        const int col = ncol0 + c * 32 + lane;
-        if (col < p.n_out) {
-          atomicAdd(p.stats + col, (double)st_s[c]);
-          atomicAdd(p.stats + p.n_out + col, (double)st_q[c]);
-        }
-      }
+      epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || blockIdx.z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + q * kStageBytes,
+                          x0 + xl0, y0 + yl0, n0 + nl0, (int)blockIdx.z);
     }
     if (det_lock) {
       __threadfence();
@@ -482,7 +412,7 @@ __global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_consta
   }
   ptx::tc_fence_before();
   __syncthreads();
-  if (warp == 2) ptx::tmem_dealloc<kTmemCols>(tmem_base);
+  if (warp == 2) ptx::tmem_dealloc<BN>(tmem_base);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -509,12 +439,11 @@ struct ConvPersistSmem {
 
 // EW = number of epilogue warps (4 or 8).  Warp w may only touch TMEM lanes 32*(w%4)..+31, so with
 // eight warps two warps share each lane quarter and split the 32-column chunks between them; that
-// doubles the epilogue throughput, which is what makes the fused BatchNorm statistics free.
-template <int BN, int MT, int STAGES, int EW, int G, bool INF>
+// doubles the epilogue throughput.
+template <int BN, int MT, int STAGES, int EW, bool INF>
 __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const __grid_constant__ TcConvParams p, int n_ntiles,
                                                                             int n_groups, int n_z, int n_work) {
   static_assert(EW == 4 || EW == 8, "4 or 8 epilogue warps");
-  static_assert(STAGES % G == 0 && STAGES / G >= 2, "at least two barrier groups");
   constexpr int kChunkGroups = EW / 4;
   extern __shared__ uint8_t smem_raw[];
   constexpr int kBBytes = BN * 128;
@@ -585,13 +514,11 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
   // Producer and MMA warps run their loops WARP-UNIFORMLY and elect one lane only around the TMA / MMA
   // issue (under a divergent `lane == 0` branch nvcc wraps every uniform-datapath instruction - UTMALDG,
   // UTCHMMA, UTCBAR - in an elect-and-retry loop).
-  // G consecutive k-blocks share ONE full/empty barrier pair: measured on B200 (scratch microbenchmarks,
-  // DESIGN.md section 3), every mbarrier wait in the MMA-issuing thread stalls it for ~105 cycles while
-  // the tensor pipe only queues ~1-2 instructions, so each wait is a ~135-cycle bubble unless the MMAs
-  // are N=256 wide (128 cycles each).  Grouping halves the number of waits per MMA.
-  constexpr int kGroups = STAGES / G;
+  // One full/empty barrier pair per k-block: sharing one pair between two k-blocks halves the ~135-cycle
+  // wait bubbles of the MMA thread (NOTES above), but measured on B200 it brought nothing and cost the
+  // 256-wide tiles 8 % (coarser refill granularity; DESIGN.md 3.3 item 2), so that variant was removed.
   if (warp == 0) {
-    int grp = 0;
+    int stage = 0;
     uint32_t phase = 0;
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
       int z, nt, g;
@@ -607,41 +534,29 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
       for (int m = 0; m < MT; ++m) tile_origin(tile0 + m, x0s[m], y0s[m], n0s[m]);
       const int ncol0 = nt * BN;
       int tp = kb0 / p.k_chunks, kc = kb0 % p.k_chunks;
-      for (int i = kb0; i < kb1; i += G) {
-        const int nk = min(G, kb1 - i);
-        ptx::mbar_wait(&empty[grp], phase ^ 1u);
+      for (int i = kb0; i < kb1; ++i) {
+        const TcTap tap = ph.taps[tp];
+        const CUtensorMap* im = &p.in_maps[tap.map];
+        ptx::mbar_wait(&empty[stage], phase ^ 1u);
         if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(&full[grp], nk * (nvalid * kABytes + kBBytes));
+          ptx::mbar_arrive_expect_tx(&full[stage], nvalid * kABytes + kBBytes);
 #pragma unroll
-          for (int j = 0; j < G; ++j) {
-            if (j < nk) {
-              const TcTap tap = ph.taps[tp];
-              const CUtensorMap* im = &p.in_maps[tap.map];
-              const int stage = grp * G + j;
-#pragma unroll
-              for (int m = 0; m < MT; ++m)
-                if (m < nvalid)
-                  ptx::tma_load_4d(sA + stage * kAStage + m * kABytes, im, &full[grp], kc * 64, x0s[m] + tap.dx, y0s[m] + tap.dy, n0s[m]);
-              ptx::tma_load_2d(sB + stage * kBBytes, &p.w_map, &full[grp], kc * 64, tap.wrow + ncol0);
-              if (++kc == p.k_chunks) { kc = 0; ++tp; }
-            }
-          }
+          for (int m = 0; m < MT; ++m)
+            if (m < nvalid)
+              ptx::tma_load_4d(sA + stage * kAStage + m * kABytes, im, &full[stage], kc * 64, x0s[m] + tap.dx, y0s[m] + tap.dy, n0s[m]);
+          ptx::tma_load_2d(sB + stage * kBBytes, &p.w_map, &full[stage], kc * 64, tap.wrow + ncol0);
         }
         __syncwarp();
-        // every lane tracks (tp, kc): only the elected lane advanced them above
-        {
-          const int adv = (i - kb0) + nk + kb0;        // absolute k-block index after this group
-          tp = adv / p.k_chunks; kc = adv - tp * p.k_chunks;
-        }
-        if (++grp == kGroups) { grp = 0; phase ^= 1u; }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
+        if (++kc == p.k_chunks) { kc = 0; ++tp; }
       }
     }
   } else if (warp == 1) {
     constexpr uint32_t idesc = ptx::make_idesc_bf16(128, BN, 0, 0);
     constexpr uint32_t kDescHi = ptx::smem_desc_hi(1024);
     const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sA), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sB), 16);
-    uint32_t a_lo = a_lo0, b_lo = b_lo0;      // descriptor low words of the current group's first stage
-    int grp = 0;
+    uint32_t a_lo = a_lo0, b_lo = b_lo0;      // descriptor low words of the current stage
+    int stage = 0;
     uint32_t phase = 0;
     int it = 0;                       // number of accumulator uses so far
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
@@ -656,30 +571,24 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
       ptx::mbar_wait(&acc_empty[as], (uint32_t)(((it >> 1) & 1) ^ 1));
       ptx::tc_fence_after();
       const uint32_t acc = tmem_base + (uint32_t)(as * kAccCols);
-      for (int i = kb0; i < kb1; i += G) {
-        const int nk = min(G, kb1 - i);
-        ptx::mbar_wait(&full[grp], phase);
+      for (int i = kb0; i < kb1; ++i) {
+        ptx::mbar_wait(&full[stage], phase);
         ptx::tc_fence_after();
         if (ptx::elect_one()) {
 #pragma unroll
-          for (int j = 0; j < G; ++j) {
-            if (j < nk) {
+          for (int m = 0; m < MT; ++m) {
+            if (m < nvalid) {
 #pragma unroll
-              for (int m = 0; m < MT; ++m) {
-                if (m < nvalid) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k)
-                    ptx::mma_bf16_ss_lohi(acc + (uint32_t)(m * BN), a_lo + (uint32_t)((j * kAStage + m * kABytes + k * 32) >> 4),
-                                          b_lo + (uint32_t)((j * kBBytes + k * 32) >> 4), kDescHi, idesc, (i + j > kb0) || (k > 0));
-                }
-              }
+              for (int k = 0; k < 4; ++k)
+                ptx::mma_bf16_ss_lohi(acc + (uint32_t)(m * BN), a_lo + (uint32_t)((m * kABytes + k * 32) >> 4),
+                                      b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc, (i > kb0) || (k > 0));
             }
           }
-          ptx::mma_commit(&empty[grp]);
+          ptx::mma_commit(&empty[stage]);
         }
         __syncwarp();
-        if (++grp == kGroups) { grp = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
-        else { a_lo += (uint32_t)((G * kAStage) >> 4); b_lo += (uint32_t)((G * kBBytes) >> 4); }
+        if (++stage == STAGES) { stage = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
+        else { a_lo += (uint32_t)(kAStage >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
       }
       if (ptx::elect_one()) ptx::mma_commit(&acc_full[as]);
       __syncwarp();
@@ -698,24 +607,6 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
     const int row0 = q * 32;
     const int xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
     int it = 0;
-    const bool do_stats = p.stats != nullptr && p.ksplit <= 1;
-    float st_s[BN / 32], st_q[BN / 32];
-#pragma unroll
-    for (int c = 0; c < BN / 32; ++c) st_s[c] = st_q[c] = 0.f;
-    int st_nt = -1;                      // N tile the register statistics belong to
-    auto flush_stats = [&]() {
-      if (st_nt < 0) return;
-#pragma unroll
-      for (int c = 0; c < BN / 32; ++c) {
-        if ((c % kChunkGroups) != cgrp) continue;
-        const int col = st_nt * BN + c * 32 + lane;
-        if (col < p.n_out) {
-          atomicAdd(p.stats + col, (double)st_s[c]);
-          atomicAdd(p.stats + p.n_out + col, (double)st_q[c]);
-        }
-        st_s[c] = st_q[c] = 0.f;
-      }
-    };
     for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
       int z, nt, g;
       decode(w, z, nt, g);
@@ -728,10 +619,6 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
       const int nvalid = min(MT, total_tiles - tile0);
       const int ncol0 = nt * BN;
       const int as = it & 1;
-      if (do_stats && nt != st_nt) {
-        flush_stats();
-        st_nt = nt;
-      }
       if (has_k) {
         ptx::mbar_wait(&acc_full[as], (uint32_t)((it >> 1) & 1));
         ptx::tc_fence_after();
@@ -756,8 +643,8 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
 #pragma unroll
             for (int j = 0; j < 32; ++j) r[j] = 0u;
           }
-          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, do_stats && has_k, lane, st_s[c], st_q[c],
-                         stage_base + ew * kStageBytes, x0 + xl0, y0 + yl0, n0 + nl0, z);
+          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + ew * kStageBytes,
+                              x0 + xl0, y0 + yl0, n0 + nl0, z);
         }
       }
       if (has_k) {
@@ -768,7 +655,6 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
         ++it;
       }
     }
-    if (do_stats) flush_stats();
     if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
   }
   ptx::tc_fence_before();
@@ -956,26 +842,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
     const int row0 = q * 32;
     const int xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
     int it = 0;
-    // BatchNorm statistics of the stored output, accumulated per lane (= column of the chunk) across this CTA's work
-    // items and flushed with fp64 atomics whenever the N tile changes
-    const bool do_stats = p.stats != nullptr && p.ksplit <= 1;
-    float st_s[BN / 32], st_q[BN / 32];
-#pragma unroll
-    for (int c = 0; c < BN / 32; ++c) st_s[c] = st_q[c] = 0.f;
-    int st_nt = -1;
-    auto flush_stats = [&]() {
-      if (st_nt < 0) return;
-#pragma unroll
-      for (int c = 0; c < BN / 32; ++c) {
-        if ((c % kChunkGroups) != cgrp) continue;
-        const int col = st_nt * BN + c * 32 + lane;
-        if (col < p.n_out) {
-          atomicAdd(p.stats + col, (double)st_s[c]);
-          atomicAdd(p.stats + p.n_out + col, (double)st_q[c]);
-        }
-        st_s[c] = st_q[c] = 0.f;
-      }
-    };
     for (int w = pair; w < n_work; w += n_pairs) {
       int z, nt, g;
       decode(w, z, nt, g);
@@ -987,10 +853,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
       const int tile0 = (g * 2 + (int)rank) * MT;
       const int ncol0 = nt * BN;
       const int as = it & 1;
-      if (do_stats && nt != st_nt) {
-        flush_stats();
-        st_nt = nt;
-      }
       if (has_k) {
         ptx::mbar_wait(&acc_full[as], (uint32_t)((it >> 1) & 1));
         ptx::tc_fence_after();
@@ -1015,8 +877,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
 #pragma unroll
             for (int j = 0; j < 32; ++j) r[j] = 0u;
           }
-          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, do_stats && has_k, lane, st_s[c], st_q[c],
-                         stage_base + ew * kStageBytes, x0 + xl0, y0 + yl0, n0 + nl0, z);
+          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + ew * kStageBytes,
+                              x0 + xl0, y0 + yl0, n0 + nl0, z);
         }
       }
       if (has_k) {
@@ -1026,7 +888,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
         ++it;
       }
     }
-    if (do_stats) flush_stats();
     if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
   }
   // neither CTA may retire while the other can still signal its barriers or read its shared memory
@@ -1365,24 +1226,23 @@ bool tc_wgrad_supported(const VgConvDesc* d) {
   return get_encode() != nullptr;
 }
 
-template <int BN, int MT, int STAGES, bool INF>
+template <int BN, int STAGES, bool INF>
 static int launch_conv_t(const TcConvParams& p, dim3 grid, cudaStream_t s) {
   static std::once_flag once;          // autograd worker threads call in concurrently
   static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_kernel<BN, MT, STAGES, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 ConvSmem<BN, MT, STAGES>::kBytes); });
+  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_kernel<BN, STAGES, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 ConvSmem<BN, STAGES>::kBytes); });
   VG_CUDA(attr_err);
-  grid.x = (unsigned)cdiv(grid.x, MT);
-  vg::Launch(grid, kTcThreads, ConvSmem<BN, MT, STAGES>::kBytes, s)(tc_conv_kernel<BN, MT, STAGES, INF>, p);
+  vg::Launch(grid, kTcThreads, ConvSmem<BN, STAGES>::kBytes, s)(tc_conv_kernel<BN, STAGES, INF>, p);
   VG_LAUNCHED();
   return VG_OK;
 }
 
-template <int BN, int MT, int STAGES, int EW, int G, bool INF>
+template <int BN, int MT, int STAGES, int EW, bool INF>
 static int launch_conv_persist_t(const TcConvParams& p, dim3 grid, cudaStream_t s) {
   static std::once_flag once;          // autograd worker threads call in concurrently
   static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_persist_kernel<BN, MT, STAGES, EW, G, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_persist_kernel<BN, MT, STAGES, EW, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  ConvPersistSmem<BN, MT, STAGES, EW>::kBytes); });
   VG_CUDA(attr_err);
   const int n_groups = (int)cdiv(grid.x, MT);
@@ -1390,7 +1250,7 @@ static int launch_conv_persist_t(const TcConvParams& p, dim3 grid, cudaStream_t 
   const int n_z = (int)grid.z;
   const long long n_work = (long long)n_groups * n_ntiles * n_z;
   const int ctas = (int)std::min<long long>(n_work, num_sms());
-  vg::Launch(ctas, 128 + 32 * EW, ConvPersistSmem<BN, MT, STAGES, EW>::kBytes, s)(tc_conv_persist_kernel<BN, MT, STAGES, EW, G, INF>, 
+  vg::Launch(ctas, 128 + 32 * EW, ConvPersistSmem<BN, MT, STAGES, EW>::kBytes, s)(tc_conv_persist_kernel<BN, MT, STAGES, EW, INF>,
       p, n_ntiles, n_groups, n_z, (int)n_work);
   VG_LAUNCHED();
   return VG_OK;
@@ -1416,15 +1276,15 @@ static int launch_conv_pair_t(const TcConvParams& p, dim3 grid, cudaStream_t s) 
 
 // the inference epilogue (activation / residual / second output) lives in its OWN instantiations: compiled into the
 // training kernels it cost them 12 % (b256 step 59.8 -> 67.3 ms: registers at the launch-bound cap, spills in the epilogue)
-template <int BN, int MT, int STAGES>
+template <int BN, int STAGES>
 static int launch_conv(const TcConvParams& p, dim3 grid, cudaStream_t s) {
   const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
-  return inf ? launch_conv_t<BN, MT, STAGES, true>(p, grid, s) : launch_conv_t<BN, MT, STAGES, false>(p, grid, s);
+  return inf ? launch_conv_t<BN, STAGES, true>(p, grid, s) : launch_conv_t<BN, STAGES, false>(p, grid, s);
 }
-template <int BN, int MT, int STAGES, int EW, int G>
+template <int BN, int MT, int STAGES, int EW>
 static int launch_conv_persist(const TcConvParams& p, dim3 grid, cudaStream_t s) {
   const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
-  return inf ? launch_conv_persist_t<BN, MT, STAGES, EW, G, true>(p, grid, s) : launch_conv_persist_t<BN, MT, STAGES, EW, G, false>(p, grid, s);
+  return inf ? launch_conv_persist_t<BN, MT, STAGES, EW, true>(p, grid, s) : launch_conv_persist_t<BN, MT, STAGES, EW, false>(p, grid, s);
 }
 template <int BN, int MT, int STAGES, int EW>
 static int launch_conv_pair(const TcConvParams& p, dim3 grid, cudaStream_t s) {
@@ -1528,22 +1388,18 @@ int tc_tune_seen(int* keys, int max_keys) {
 }
 
 static int pick_bn(int n_out) {
-  static int forced = -1;
-  if (forced < 0) {
-    const char* e = getenv("VG_TC_BN");
-    forced = e ? atoi(e) : 0;
-  }
-  if (forced && n_out % forced == 0) return forced;
   if (n_out % 256 == 0) return 256;
   if (n_out % 128 == 0) return 128;
   return 64;
 }
 
+// kernel-form heuristic of tc_conv_run (a tile-table form overrides it)
+constexpr int kPersistMinItemsPerSm64 = 6;   // 64-wide tiles go persistent from this many work items per SM on
+constexpr int kPairMinBN = 128;              // CTA pairs for 128- and 256-wide tiles; 64-wide tiles gain nothing (DESIGN.md 3.1)
+
 // dgrad=false: y = conv(x).  dgrad=true: dx from dy.  `in` is the tensor being read.
 int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpack, const float* bias, const float* colscale,
-                const float* sigma, int sigma_group_n, void* out, int out_dtype, double* stats, bool* stats_fused, cudaStream_t s,
-                const VgConvEpilogue* ep) {
-  if (stats_fused) *stats_fused = false;
+                const float* sigma, int sigma_group_n, void* out, int out_dtype, cudaStream_t s, const VgConvEpilogue* ep) {
   TcConvParams p;
   memset(&p, 0, sizeof(p));
   // pattern: which side is the coarse grid
@@ -1566,7 +1422,6 @@ int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpa
     p.act_slope = ep->act_slope; p.residual = ep->residual; p.out2 = ep->y2;
     p.post_scale = ep->post_scale; p.post_shift = ep->post_shift; p.post_slope = ep->post_slope;
   }
-  p.stats = nullptr;
   int nphase = 1;
   if (gather) {
     p.gw = out_w; p.gh = out_h; p.gn = d->n; p.os = 1;
@@ -1631,8 +1486,8 @@ int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpa
   // kernel variant: persistent CTAs (double-buffered accumulator, MT pixel tiles share each staged weight
   // tile) when there is enough work; one-shot CTAs (two resident per SM) for small problems and split-K.
   // Measured on B200 (scripts/sweep_conv.py): a persistent single-tile CTA loses to two co-resident
-  // one-shot CTAs, and multi-tile CTAs without the double-buffered accumulator are slower still
-  // (128->128 @96: 897 -> 769 TFLOP/s), so those stay opt-in (VG_TC_MT=1).
+  // one-shot CTAs, and one-shot CTAs of two pixel tiles (no double-buffered accumulator) were slower still
+  // (128->128 @96: 897 -> 769 TFLOP/s) and were removed.
   // TMA-store epilogue (VG_TC_TMA_STORE, default 2): bf16 outputs without split-K and without the inference epilogue leave
   // the staging buffers as cp.async.bulk.tensor stores - 1: gather-type launches only (output on the GEMM's own pixel grid),
   // 2: also the scatter launches (one strided output map per phase), 0: the manual coalesced stores.  Measured on B200
@@ -1649,43 +1504,22 @@ int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpa
         return rc;
     p.tma_store = 1;
   }
-  static int mt_on = -1, persist = -1, mt_min = -1, fuse_stats = -1;
-  if (mt_on < 0) { const char* e = getenv("VG_TC_MT"); mt_on = (e && atoi(e)) ? 1 : 0; }
-  if (persist < 0) { const char* e = getenv("VG_TC_PERSIST"); persist = e ? atoi(e) : 1; }
-  if (mt_min < 0) { const char* e = getenv("VG_TC_MT_MIN"); mt_min = e ? atoi(e) : 6; }
-  if (fuse_stats < 0) { const char* e = getenv("VG_TC_FUSE_STATS"); fuse_stats = e ? atoi(e) : 0; }
   const long long ctas1 = (long long)grid.x * grid.y * grid.z;
-  const bool big = mt_on && p.ksplit == 1 && ctas1 >= 6LL * num_sms();
   // 256-wide tiles go persistent as soon as there is more than one work item per SM (288 tiles of the 24x24 layers at
   // batch 64 ran as one-shot CTAs without epilogue overlap: 38-85 us for 31 us of tensor work)
-  const bool heur_persist = persist && !(g_det.on && p.ksplit > 1) &&       // deterministic split-K: the one-shot kernel takes turns
-                           ((BN == 256 && ctas1 > (long long)num_sms()) ||
-                                       // 128-wide: the CTA-pair kernel (1000+ TFLOP/s) from two work items per pair on; below 6 x SMs tiles
-                                       // these layers ran as one-shot CTAs (G 128->128 @48 at 32 images: 496 TFLOP/s)
-                                       (BN == 128 && ctas1 >= 2LL * num_sms()) ||
-                                       (BN == 64 && ctas1 >= 2LL * num_sms() && ctas1 >= (long long)mt_min * num_sms()));
+  const bool heur_persist = !(g_det.on && p.ksplit > 1) &&       // deterministic split-K: the one-shot kernel takes turns
+                            ((BN == 256 && ctas1 > (long long)num_sms()) ||
+                             // 128-wide: the CTA-pair kernel (1000+ TFLOP/s) from two work items per pair on; below 6 x SMs tiles
+                             // these layers ran as one-shot CTAs (G 128->128 @48 at 32 images: 496 TFLOP/s)
+                             (BN == 128 && ctas1 >= 2LL * num_sms()) ||
+                             (BN == 64 && ctas1 >= (long long)kPersistMinItemsPerSm64 * num_sms()));
   // a tile-table entry overrides the form (split-K launches keep the heuristic: only the one-shot kernel was tuned for them)
   const int form = p.ksplit > 1 ? kFormAuto : tuned.form;
   const bool use_persist = form == kFormAuto ? heur_persist : (form != kFormOneShot);
-  // BatchNorm statistics of the output can be accumulated by the epilogue warps of the 8-warp persistent
-  // kernels (parity-tested), but it is OPT-IN (VG_TC_FUSE_STATS=1): measured on B200 the per-chunk smem
-  // transposes cost the L2/smem-bound main loop more (+35 % per launch with 8 epilogue warps, +60 % with
-  // 4) than the separate 20 us statistics kernel they replace.
-  // Round 2 replaced the shared-memory transpose by a 31-shuffle recursive halving per 32 x 32 chunk and enabled it in
-  // every kernel form - measured on B200 (scripts/sweep_conv.py, batch 64) it is STILL a loss: 64->64 @96 74.9 -> 163 us,
-  // 128->128 @96 151 -> 217 us, 512->512 @24 110 -> 125 us, whole step 63.7 -> 68.2 ms, against the 17 us streaming
-  // statistics kernel it replaces: the epilogue warps are the bottleneck of the short-reduction layers and ~350 extra
-  // instructions per chunk double their work.  Kept opt-in (VG_TC_FUSE_STATS=1) and parity-tested.
-  if (fuse_stats && !g_det.on && stats != nullptr && p.ksplit == 1 && n_out % 32 == 0 && p.n_store != 1) {
-    p.stats = stats;
-    if (stats_fused) *stats_fused = true;
-  }
   // CTA pairs (cta_group::2) halve the per-SM shared-memory operand reads that bound the narrow tiles
-  static int pair_on = -1;
-  if (pair_on < 0) { const char* e = getenv("VG_TC_PAIR"); pair_on = e ? atoi(e) : 6; }   // bit0: BN=64, bit1: BN=128, bit2: BN=256
-  if (use_persist && form != kFormPersist && (pair_on || form == kFormPair) && p.n_store != 1) {
+  if (use_persist && p.n_store != 1 && (form == kFormPair || (form == kFormAuto && BN >= kPairMinBN))) {
     const int mt = BN == 64 ? 4 : (BN == 128 ? 2 : 1);
-    if (grid.x % (2 * mt) == 0 && (form == kFormPair || (pair_on & (BN == 64 ? 1 : (BN == 128 ? 2 : 4))))) {
+    if (grid.x % (2 * mt) == 0) {
       if ((rc = make_weight_map(&p.w_map, wpack, (long long)k * k * n_out, in_c, BN / 2))) return rc;
       switch (BN) {
         case 64: return launch_conv_pair<64, 4, 3, 4>(p, grid, s);
@@ -1695,27 +1529,21 @@ int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpa
       }
     }
   }
-  static int grp2 = -1;
-  if (grp2 < 0) { const char* e = getenv("VG_TC_GROUP"); grp2 = e ? (atoi(e) == 2) : 0; }
   // 64-wide tiles are EPILOGUE-bound (9 k-blocks of N=64 MMAs per 128 x 64 outputs).  Eight epilogue warps instead of four
-  // (VG_TC_EW64=82: <64,2,4,8>) measured NO gain on B200 (64->64 @96: 74.4 vs 74.9 us): the bound was the store path
+  // (<64,2,4,8>) measured NO gain on B200 (64->64 @96: 74.4 vs 74.9 us) and were removed: the bound was the store path
   // (32 lines per store instruction), addressed by the staged, coalesced stores of epilogue_chunk.
-  static int ew64 = -1;
-  if (ew64 < 0) { const char* e = getenv("VG_TC_EW64"); ew64 = e ? atoi(e) : 4; }
   if (use_persist) {
     switch (BN) {
-      case 64:
-        if (ew64 == 82) return launch_conv_persist<64, 2, 4, 8, 1>(p, grid, s);
-        return launch_conv_persist<64, 4, 3, 4, 1>(p, grid, s);
-      case 128: return grp2 ? launch_conv_persist<128, 2, 4, 8, 2>(p, grid, s) : launch_conv_persist<128, 2, 4, 8, 1>(p, grid, s);
-      case 256: return grp2 ? launch_conv_persist<256, 1, 4, 8, 2>(p, grid, s) : launch_conv_persist<256, 1, 4, 8, 1>(p, grid, s);
+      case 64: return launch_conv_persist<64, 4, 3, 4>(p, grid, s);
+      case 128: return launch_conv_persist<128, 2, 4, 8>(p, grid, s);
+      case 256: return launch_conv_persist<256, 1, 4, 8>(p, grid, s);
       default: break;
     }
   }
   switch (BN) {
-    case 64: rc = big ? launch_conv<64, 2, 4>(p, grid, s) : launch_conv<64, 1, 4>(p, grid, s); break;
-    case 128: rc = big ? launch_conv<128, 2, 4>(p, grid, s) : launch_conv<128, 1, 3>(p, grid, s); break;
-    case 256: rc = launch_conv<256, 1, 4>(p, grid, s); break;
+    case 64: rc = launch_conv<64, 4>(p, grid, s); break;
+    case 128: rc = launch_conv<128, 3>(p, grid, s); break;
+    case 256: rc = launch_conv<256, 4>(p, grid, s); break;
     default: set_error("unsupported BN %d", BN); return VG_EUNSUPPORTED;
   }
   if (rc == VG_OK && p.det_split_stride != 0)
@@ -1744,9 +1572,7 @@ int tc_wgrad_run(const VgConvDesc* d, const void* x, const void* dy, float* dw, 
   p.n_boxes = p.tiles_x * p.tiles_y * p.tiles_n;
   // 1x1 convolutions / Linear layers: torch layout [c_u][c_s] already has c_s contiguous, so the epilogue's per-lane
   // reductions are coalesced (32 lanes = 32 consecutive c_s) and the scratch + memset + unpack round trip is skipped
-  static int direct11 = -1;
-  if (direct11 < 0) { const char* e = getenv("VG_WGRAD_DIRECT_1X1"); direct11 = e ? atoi(e) : 1; }
-  p.packed = workspace != nullptr && (tmp.ntaps > 1 || (!direct11 && !acc_only));
+  p.packed = workspace != nullptr && tmp.ntaps > 1;
   p.dw = (p.packed || acc_only) ? workspace : dw;
   const size_t welems = (size_t)k * k * cs * cu;
   if (p.packed && !acc_only) VG_CUDA(cudaMemsetAsync(workspace, 0, welems * sizeof(float), s));
