@@ -247,7 +247,7 @@ CONV_CASES_TC = [
     (512, 512, 3, 1, 1, False, 2, 6),
     (64, 1, 3, 1, 1, False, 2, 16),        # single output channel through the tensor-core kernel
     (64, 1, 3, 1, 1, False, 3, 24),
-    (64, 128, 3, 1, 1, False, 16, 96),     # enough tiles for the persistent 8-epilogue-warp kernel
+    (64, 128, 3, 1, 1, False, 16, 96),     # enough tiles for the CTA-pair kernel: forward runs pair<128,2,4,8>
     (128, 256, 3, 1, 1, False, 8, 96),     # persistent <256,1,4,8>
     (64, 64, 3, 1, 1, False, 16, 96),      # persistent <64,4,3,4>
 ]
