@@ -206,7 +206,6 @@ __global__ void __launch_bounds__(kThreads, 2) bn_stream_kernel(const __grid_con
       __syncwarp();
       if (++stage == ST) { stage = 0; phase ^= 1u; }
     }
-    vg::pdl_tail_trigger();
     return;
   }
 
@@ -386,7 +385,6 @@ __global__ void __launch_bounds__(kThreads, 2) bn_stream_kernel(const __grid_con
     if (lane == 0) ptx::mbar_arrive(&empty[stage]);
     if (++stage == ST) { stage = 0; phase ^= 1u; }
   }
-  vg::pdl_tail_trigger();
 
   if (ModeTraits<MODE>::kReduce) {
     // per-channel block reduction through the (now idle) ring, then one fp64 atomic per (block, channel, quantity)

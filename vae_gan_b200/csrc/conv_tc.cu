@@ -17,7 +17,11 @@
 //     warps 4.. = epilogue (tcgen05.ld -> bias / Dropout2d column scale -> bf16|f32 -> global).
 //   Three forms, chosen per layer by tc_conv_run: one-shot CTAs (tc_conv_kernel, small problems and split-K),
 //   persistent CTAs with a double-buffered TMEM accumulator (tc_conv_persist_kernel), and persistent CTA
-//   pairs issuing M=256 cta_group::2 MMAs (tc_conv_pair_kernel, 128/256-wide tiles).
+//   pairs issuing M=256 cta_group::2 MMAs (tc_conv_pair_kernel, 128/256-wide tiles).  The persist and pair
+//   kernels are one body (conv_persistent, CTAs per MMA as a template argument), and all three forms run each
+//   work item through the same producer, MMA and epilogue pieces (load_item, mma_item, drain_tile).  Every
+//   tcgen05 kernel, tc_wgrad_kernel included, takes its shared-memory layout from TcSmem (the host reads the
+//   launch size from the same type) and shares tc_prologue / tc_teardown.
 //
 // tc_wgrad_kernel: dW[128 = 2 x 64 (tap, c_s chunk)][BN = c_u tile] += S^T . U over a range of
 //   64-pixel boxes (split-K across CTAs, fp32 atomics into the torch-layout gradient).  Both
@@ -93,14 +97,114 @@ constexpr int kTcThreads = 256;
 constexpr int kABytes = 128 * 128;   // 128 rows x 64 bf16
 constexpr int kStageBytes = 32 * 64;  // per epilogue warp: 32 rows x 32 bf16 of one output chunk (coalescing transpose)
 
+// Dynamic shared memory of a tcgen05 kernel; the host takes kBytes for the launch, the kernel takes the pointers.
+// At a 1024-byte boundary (the 128-byte swizzle atoms): a STAGES-deep ring of A stages (A_BYTES) and B stages (B_BYTES),
+// the ring's full[STAGES] / empty[STAGES] mbarriers, NACC accumulator mbarriers, the TMEM address slot and EW per-warp
+// epilogue staging buffers.  The staging buffers are 512-byte aligned: their XOR pattern is then exactly TMA's 64-byte
+// swizzle (absolute address bits).
+template <int STAGES, int A_BYTES, int B_BYTES, int NACC, int EW>
+struct TcSmem {
+  static constexpr int kStages = STAGES, kA = A_BYTES, kB = B_BYTES;
+  static constexpr int kBytes =
+      1024 + STAGES * (A_BYTES + B_BYTES) + (2 * STAGES + NACC) * 8 + 16 + (EW > 0 ? 16 + 512 + EW * kStageBytes : 0);
+  uint8_t* a;
+  uint8_t* b;
+  uint64_t* full;
+  uint64_t* empty;
+  uint64_t* acc;
+  uint32_t* tmem_slot;
+  uint8_t* stage;
+  __device__ explicit TcSmem(uint8_t* raw) {
+    a = raw + ((1024u - (ptx::smem_u32(raw) & 1023u)) & 1023u);
+    b = a + STAGES * A_BYTES;
+    full = reinterpret_cast<uint64_t*>(b + STAGES * B_BYTES);
+    empty = full + STAGES;
+    acc = empty + STAGES;
+    tmem_slot = reinterpret_cast<uint32_t*>(acc + NACC);
+    stage = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 511) & ~(uintptr_t)511);
+  }
+};
+
+// one-shot form: one accumulator barrier, four epilogue warps
 template <int BN, int STAGES>
-struct ConvSmem {
-  static constexpr int kBBytes = BN * 128;
-  static constexpr int kBytes = STAGES * (kABytes + kBBytes) + (2 * STAGES + 1) * 8 + 16 + 1024 + 4 * kStageBytes + 16 + 512;
+using ConvSmem = TcSmem<STAGES, kABytes, BN * 128, 1, 4>;
+// persistent forms: MT pixel tiles per A stage, a CTA of a pair (CTAS = 2) stages half of the weight tile; acc_full[2], acc_empty[2]
+template <int CTAS, int BN, int MT, int STAGES, int EW>
+using ConvPersistSmem = TcSmem<STAGES, MT * kABytes, (BN / CTAS) * 128, 4, EW>;
+// weight gradient: one stage = two S boxes and NB U boxes of 8 KB
+template <int NB, int STAGES>
+using WgradSmem = TcSmem<STAGES, (2 + NB) * 8192, 0, 1, 0>;
+
+// Set-up of every tcgen05 kernel: warp 0 prefetches two tensor-map descriptors, warp 1 initialises the ring barriers and
+// (init_acc) the accumulator barriers, warp 2 allocates TMEM_COLS TMEM columns (for both CTAs of a pair when CTAS == 2).
+// The CTA - or the pair - then synchronises, so every barrier of both CTAs exists before anyone signals it.  All of this
+// overlaps the previous kernel's tail: it runs before pdl_entry() and touches no global memory.  Returns the TMEM base.
+template <int CTAS, int TMEM_COLS, class Smem, class InitAcc>
+__device__ __forceinline__ uint32_t tc_prologue(const Smem& sm, const CUtensorMap* map0, const CUtensorMap* map1, InitAcc init_acc) {
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (warp == 0 && lane == 0) {
+    ptx::prefetch_tmap(map0);
+    ptx::prefetch_tmap(map1);
+  }
+  if (warp == 1 && lane == 0) {
+    for (int s = 0; s < Smem::kStages; ++s) {
+      ptx::mbar_init(&sm.full[s], 1);
+      ptx::mbar_init(&sm.empty[s], 1);
+    }
+    init_acc();
+    ptx::fence_barrier_init();
+  }
+  if (warp == 2) {
+    if constexpr (CTAS == 2) ptx::tmem_alloc_pair<TMEM_COLS>(sm.tmem_slot);
+    else ptx::tmem_alloc<TMEM_COLS>(sm.tmem_slot);
+  }
+  ptx::tc_fence_before();
+  if constexpr (CTAS == 2) ptx::cluster_sync();
+  else __syncthreads();
+  ptx::tc_fence_after();
+  vg::pdl_entry();
+  return *sm.tmem_slot;
+}
+
+// Neither the CTA's warps nor the pair's other CTA may still use its TMEM, signal its barriers or read its shared memory
+// when it frees the TMEM and retires.
+template <int CTAS, int TMEM_COLS>
+__device__ __forceinline__ void tc_teardown(uint32_t tmem_base) {
+  ptx::tc_fence_before();
+  if constexpr (CTAS == 2) ptx::cluster_sync();
+  else __syncthreads();
+  if ((threadIdx.x >> 5) == 2) {
+    if constexpr (CTAS == 2) ptx::tmem_dealloc_pair<TMEM_COLS>(tmem_base);
+    else ptx::tmem_dealloc<TMEM_COLS>(tmem_base);
+  }
+}
+
+// origin of pixel tile t (a TW x TH x TN box of the GEMM pixel grid; x fastest, then y, then image)
+struct Tile { int x0, y0, n0; };
+template <class P>
+__device__ __forceinline__ Tile tile_origin(const P& p, int t) {
+  const int tx = t % p.tiles_x; t /= p.tiles_x;
+  const int ty = t % p.tiles_y;
+  const int tn = t / p.tiles_y;
+  return Tile{tx * p.TW, ty * p.TH, tn * p.TN};
+}
+
+// a role warp's position in the operand ring
+template <class Smem>
+struct RingPos {
+  int stage = 0;
+  uint32_t phase = 0;
+  __device__ __forceinline__ bool next() {     // true when the ring wraps
+    if (++stage < Smem::kStages) return false;
+    stage = 0;
+    phase ^= 1u;
+    return true;
+  }
 };
 
 // Finishes one 32-column chunk of one accumulator row per thread: 1/sigma, bias, Dropout2d column scale, store
-// (bf16 / fp32 / split-K vector reductions / single channel).
+// (bf16 / fp32 / split-K vector reductions / single channel).  z is the work item's output phase, or its k-split when
+// p.ksplit > 1 (the bias is added by split 0 only).
 //
 // bf16 outputs go through `stage` (a 2 KB per-warp shared-memory buffer) when it is given: lane = pixel row holds 64 B of
 // consecutive channels, so a direct 16-byte store per lane touches 32 different 128-byte lines per instruction - the
@@ -108,10 +212,10 @@ struct ConvSmem {
 // layers).  The warp writes its 32 x 64 B block into shared memory (XOR-swizzled 16-byte units, conflict-free both ways),
 // reads it back transposed and stores with FOUR consecutive lanes covering one row's 64 bytes: 8 lines per instruction.
 template <bool INF>
-__device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint32_t (&r)[32], bool valid, bool add_bias,
-                                               long long opix, int gn, int ncol, bool first_chunk, uint8_t* stage = nullptr,
-                                               int sx = 0, int sy = 0, int sn = 0, int out_phase = 0) {
+__device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint32_t (&r)[32], bool valid, long long opix, int gn,
+                                               int ncol, bool first_chunk, uint8_t* stage, int sx, int sy, int sn, int z) {
   const int lane = threadIdx.x & 31;
+  const bool add_bias = p.ksplit <= 1 || z == 0;
   float v[32];
 #pragma unroll
   for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(r[j]);
@@ -158,7 +262,7 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint
       ptx::fence_proxy_async_smem();
       __syncwarp();
       if (lane == 0) {
-        ptx::tma_store_4d(&p.out_maps[out_phase], stage, ncol, sx, sy, sn);
+        ptx::tma_store_4d(&p.out_maps[z], stage, ncol, sx, sy, sn);
         ptx::bulk_commit_group();
       }
       __syncwarp();
@@ -236,8 +340,8 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint
       // Linear layers' one-shot CTAs spent most of their time issuing them; n_out % 64 == 0 keeps them aligned)
       float* o = reinterpret_cast<float*>(p.out) + opix * p.n_out + ncol;
       if (p.det_split_stride != 0) {
-        // deterministic mode: this split's partial tile goes to its own scratch slab (one-shot kernel: split = blockIdx.z)
-        o += (long long)blockIdx.z * p.det_split_stride;
+        // deterministic mode: this split's partial tile goes to its own scratch slab
+        o += (long long)z * p.det_split_stride;
 #pragma unroll
         for (int j = 0; j < 32; j += 4) *reinterpret_cast<float4*>(o + j) = make_float4(v[j], v[j + 1], v[j + 2], v[j + 3]);
       } else {
@@ -269,224 +373,243 @@ __device__ __forceinline__ void epilogue_chunk(const TcConvParams& p, const uint
 // ------------------------------------------------------------------------------------------
 // forward / dgrad implicit GEMM
 // ------------------------------------------------------------------------------------------
-// one-shot form: one CTA per (128-pixel tile, N tile, phase | k-split)
-template <int BN, int STAGES, bool INF>
-__global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_constant__ TcConvParams p) {
-  extern __shared__ uint8_t smem_raw[];
-  constexpr int kBBytes = BN * 128;
-  const uint32_t raw_addr = ptx::smem_u32(smem_raw);
-  uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + STAGES * kABytes;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sB + STAGES * kBBytes);
-  uint64_t* empty = full + STAGES;
-  uint64_t* tmem_full = empty + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
-  // 512-byte aligned: the staging buffers' XOR pattern is then exactly TMA's 64-byte swizzle (absolute address bits)
-  uint8_t* stage_base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 511) & ~(uintptr_t)511);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : blockIdx.z];
-  const int ntaps = ph.ntaps;
-  const int kb0 = p.ksplit > 1 ? (int)blockIdx.z * p.k_per_split : 0;
-  const int kb1 = p.ksplit > 1 ? min(ntaps * p.k_chunks, kb0 + p.k_per_split) : ntaps * p.k_chunks;
-  const int num_k = max(0, kb1 - kb0);
-  int x0, y0, n0;
-  {
-    int t = blockIdx.x;
-    const int tx = t % p.tiles_x; t /= p.tiles_x;
-    const int ty = t % p.tiles_y;
-    const int tn = t / p.tiles_y;
-    x0 = tx * p.TW; y0 = ty * p.TH; n0 = tn * p.TN;
-  }
-  const int ncol0 = blockIdx.y * BN;
-
-  if (warp == 0 && lane == 0) {
-    ptx::prefetch_tmap(&p.w_map);
-    ptx::prefetch_tmap(&p.in_maps[0]);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    ptx::mbar_init(tmem_full, 1);
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) ptx::tmem_alloc<BN>(tmem_slot);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  vg::pdl_entry();   // barriers, TMEM and descriptor prefetch above overlap the previous kernel's tail; nothing above touches global memory
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (num_k > 0) {
-    // both role warps loop warp-uniformly and elect a lane only around the TMA / MMA issue (a divergent
-    // `lane == 0` branch makes nvcc wrap every uniform-datapath instruction in an elect-and-retry loop)
-    if (warp == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      int tp = kb0 / p.k_chunks, kc = kb0 % p.k_chunks;
-      for (int i = kb0; i < kb1; ++i) {
-        const TcTap tap = ph.taps[tp];
-        const CUtensorMap* im = &p.in_maps[tap.map];
-        ptx::mbar_wait(&empty[stage], phase ^ 1u);
-        if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(&full[stage], kABytes + kBBytes);
-          ptx::tma_load_4d(sA + stage * kABytes, im, &full[stage], kc * 64, x0 + tap.dx, y0 + tap.dy, n0);
-          ptx::tma_load_2d(sB + stage * kBBytes, &p.w_map, &full[stage], kc * 64, tap.wrow + ncol0);
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-        if (++kc == p.k_chunks) { kc = 0; ++tp; }
-      }
-    } else if (warp == 1) {
-      constexpr uint32_t idesc = ptx::make_idesc_bf16(128, BN, 0, 0);
-      constexpr uint32_t kDescHi = ptx::smem_desc_hi(1024);
-      const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sA), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sB), 16);
-      uint32_t a_lo = a_lo0, b_lo = b_lo0;      // descriptor low words of the current stage
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int i = 0; i < num_k; ++i) {
-        ptx::mbar_wait(&full[stage], phase);
-        ptx::tc_fence_after();
-        if (ptx::elect_one()) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            ptx::mma_bf16_ss_lohi(tmem_base, a_lo + (uint32_t)((k * 32) >> 4), b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc,
-                                  (i | k) != 0);
-          ptx::mma_commit(&empty[stage]);
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
-        else { a_lo += (uint32_t)(kABytes >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
-      }
-      if (ptx::elect_one()) ptx::mma_commit(tmem_full);
-      __syncwarp();
-      vg::pdl_tail_trigger();
-    }
-  }
-
-  if (warp >= 4) {
-    const int q = warp - 4;
-    const int row = q * 32 + lane;
-    const int xl = row & (p.TW - 1);
-    const int yl = (row >> p.tw_log2) & (p.TH - 1);
-    const int nl = row >> (p.tw_log2 + p.th_log2);
-    // first pixel of this warp's 32-row quarter inside the tile: origin of its TMA-store sub-box
-    const int row0 = q * 32;
-    const int xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
-    if (num_k > 0) {
-      ptx::mbar_wait(tmem_full, 0);
-      ptx::tc_fence_after();
-    }
-    // deterministic split-K: this split's reductions go after those of split z - 1 of the same output tile
-    int* const det_lock = (p.det_locks != nullptr && p.ksplit > 1) ? p.det_locks + (blockIdx.y * gridDim.x + blockIdx.x) : nullptr;
-    if (det_lock) {
-      if (lane == 0) det_wait_turn(det_lock, (int)blockIdx.z);
-      __syncwarp();
-    }
-    const int gx = x0 + xl, gy = y0 + yl, gn = n0 + nl;
-    const bool valid = gx < p.gw && gy < p.gh && gn < p.gn && !(p.ksplit > 1 && num_k == 0 && p.det_split_stride == 0);
-    const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
-#pragma unroll
-    for (int c = 0; c < BN / 32; ++c) {
-      const int c0 = c * 32;
-      uint32_t r[32];
-      if (num_k > 0) {
-        ptx::tmem_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)c0, r);
-        ptx::tmem_ld_wait();
-      } else {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) r[j] = 0u;
-      }
-      epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || blockIdx.z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + q * kStageBytes,
-                          x0 + xl0, y0 + yl0, n0 + nl0, (int)blockIdx.z);
-    }
-    if (det_lock) {
-      __threadfence();
-      asm volatile("bar.sync 2, 128;" ::: "memory");      // the four epilogue warps
-      if (warp == 4 && lane == 0) det_publish_turn(det_lock, (int)blockIdx.z + 1 == p.ksplit ? 0 : (int)blockIdx.z + 1);
-    }
-    if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 2) ptx::tmem_dealloc<BN>(tmem_base);
-}
-
-// ------------------------------------------------------------------------------------------
 // NOTES (measured on B200, round 1; microbenchmarks in scripts/microbench/, numbers in DESIGN.md section 3):
 //  * a tcgen05.mma (M=128, K=16, SS mode) takes max(N/2, 32 + N/4) cycles - the operands are re-read from
 //    shared memory at 128 B/cycle - so N=64 tiles cap at 67 % of the tensor peak, N>=128 can reach it;
 //  * the tensor pipe queues only ~1-2 instructions and every mbarrier wait stalls the issuing thread for
 //    ~105 cycles: one wait per k-block costs a ~135-cycle bubble unless the queued MMAs are N=256 wide;
+//    sharing one full/empty barrier pair between two k-blocks halves those waits but measured nothing in the
+//    real kernel and cost the 256-wide tiles 8 % (coarser refill granularity; DESIGN.md 3.3 item 2);
 //  * under a divergent `lane == 0` branch nvcc wraps each UTCHMMA/UTMALDG in an elect-and-retry loop and
 //    rebuilding 64-bit descriptors costs ~14 uniform instructions per MMA: the role warps therefore run
 //    warp-uniformly, elect only around the issue, and advance 32-bit descriptor halves by adds;
 //  * the chip is power-capped under tensor load (SM clock 1.3-1.5 GHz), so removing loads, stores or waits
 //    buys cycles but little time; what pays is fewer shared-memory/L2 bytes per FLOP (CTA pairs below).
 //
-// persistent variant: one CTA per SM loops over work items (phase|k-split, N tile, group of MT
-// pixel tiles); the TMEM accumulator is double-buffered so the epilogue of item i overlaps the
-// main loop of item i+1, and the MT pixel tiles of an item share every staged weight tile.
-// ------------------------------------------------------------------------------------------
-template <int BN, int MT, int STAGES, int EW>
-struct ConvPersistSmem {
-  static constexpr int kBBytes = BN * 128;
-  static constexpr int kBytes = STAGES * (MT * kABytes + kBBytes) + (2 * STAGES + 4) * 8 + 16 + 1024 + EW * kStageBytes + 16 + 512;
+// The three forms share the per-item pieces below: conv_slice (which k-blocks an item reduces), load_item (producer warp),
+// mma_item (MMA warp) and drain_tile (epilogue warps).
+
+// k-blocks [kb0, kb1) of slice z - an output phase, or a k-split when p.ksplit > 1 - and the tap table they read
+__device__ __forceinline__ const TcPhase& conv_slice(const TcConvParams& p, int z, int& kb0, int& kb1) {
+  const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
+  const int total = ph.ntaps * p.k_chunks;
+  if (p.ksplit > 1) { kb0 = z * p.k_per_split; kb1 = min(total, kb0 + p.k_per_split); }
+  else { kb0 = 0; kb1 = total; }
+  if (kb1 < kb0) kb1 = kb0;
+  return ph;
+}
+
+// Producer warp, one work item: k-blocks [kb0, kb1) into the ring.  A k-block is the A boxes of the first `nvalid` of the
+// CTA's MT pixel tiles (at the tap's shift) and the weight tile from row tap.wrow + wrow0.  In a CTA pair (CTAS == 2) both
+// CTAs count their bytes on the leader's full barrier, which the leader (rank 0) arms for both.
+template <int CTAS, int MT, class Smem>
+__device__ __forceinline__ void load_item(const TcConvParams& p, const TcPhase& ph, int kb0, int kb1, const Tile (&t)[MT], int nvalid,
+                                          int wrow0, uint32_t rank, const Smem& sm, RingPos<Smem>& pos) {
+  int tp = kb0 / p.k_chunks, kc = kb0 % p.k_chunks;
+  for (int i = kb0; i < kb1; ++i) {
+    const TcTap tap = ph.taps[tp];
+    const CUtensorMap* im = &p.in_maps[tap.map];
+    ptx::mbar_wait(&sm.empty[pos.stage], pos.phase ^ 1u);
+    if (ptx::elect_one()) {
+      uint8_t* a = sm.a + pos.stage * Smem::kA;
+      uint8_t* b = sm.b + pos.stage * Smem::kB;
+      if constexpr (CTAS == 2) {
+        if (rank == 0) ptx::mbar_arrive_expect_tx(&sm.full[pos.stage], 2 * (Smem::kA + Smem::kB));
+        const uint32_t bar = ptx::mapa(ptx::smem_u32(&sm.full[pos.stage]), 0);
+#pragma unroll
+        for (int m = 0; m < MT; ++m)
+          ptx::tma_load_4d_pair(a + m * kABytes, im, bar, kc * 64, t[m].x0 + tap.dx, t[m].y0 + tap.dy, t[m].n0);
+        ptx::tma_load_2d_pair(b, &p.w_map, bar, kc * 64, tap.wrow + wrow0);
+      } else {
+        ptx::mbar_arrive_expect_tx(&sm.full[pos.stage], nvalid * kABytes + Smem::kB);
+#pragma unroll
+        for (int m = 0; m < MT; ++m)
+          if (m < nvalid)
+            ptx::tma_load_4d(a + m * kABytes, im, &sm.full[pos.stage], kc * 64, t[m].x0 + tap.dx, t[m].y0 + tap.dy, t[m].n0);
+        ptx::tma_load_2d(b, &p.w_map, &sm.full[pos.stage], kc * 64, tap.wrow + wrow0);
+      }
+    }
+    __syncwarp();
+    pos.next();
+    if (++kc == p.k_chunks) { kc = 0; ++tp; }
+  }
+}
+
+// tcgen05.commit to `bar` (of both CTAs of a pair) once the MMAs issued so far have completed
+template <int CTAS>
+__device__ __forceinline__ void commit_to(uint64_t* bar) {
+  if constexpr (CTAS == 2) ptx::mma_commit_pair(bar, 3);
+  else ptx::mma_commit(bar);
+}
+
+// MMA warp, one work item: num_k k-blocks from the ring into the accumulator at TMEM address `acc` (pixel tile m at column
+// m * BN; M = 256 over both CTAs of a pair, issued by the leader alone), releasing each stage as its MMAs complete.
+// a_lo / b_lo are the descriptor low words of the ring position's stage (a_lo0 / b_lo0: stage 0).
+template <int CTAS, int BN, int MT, class Smem>
+__device__ __forceinline__ void mma_item(uint32_t acc, int num_k, int nvalid, const Smem& sm, RingPos<Smem>& pos, uint32_t a_lo0,
+                                         uint32_t b_lo0, uint32_t& a_lo, uint32_t& b_lo) {
+  constexpr uint32_t idesc = ptx::make_idesc_bf16(128 * CTAS, BN, 0, 0);
+  constexpr uint32_t kDescHi = ptx::smem_desc_hi(1024);
+  for (int i = 0; i < num_k; ++i) {
+    ptx::mbar_wait(&sm.full[pos.stage], pos.phase);
+    ptx::tc_fence_after();
+    if (ptx::elect_one()) {
+#pragma unroll
+      for (int m = 0; m < MT; ++m) {
+        if (m < nvalid) {
+#pragma unroll
+          for (int k = 0; k < 4; ++k) {
+            const uint32_t d = acc + (uint32_t)(m * BN), a = a_lo + (uint32_t)((m * kABytes + k * 32) >> 4),
+                           b = b_lo + (uint32_t)((k * 32) >> 4);
+            if constexpr (CTAS == 2) ptx::mma_bf16_ss_pair_lohi(d, a, b, kDescHi, idesc, (i | k) != 0);
+            else ptx::mma_bf16_ss_lohi(d, a, b, kDescHi, idesc, (i | k) != 0);
+          }
+        }
+      }
+      commit_to<CTAS>(&sm.empty[pos.stage]);
+    }
+    __syncwarp();
+    if (pos.next()) { a_lo = a_lo0; b_lo = b_lo0; }
+    else { a_lo += (uint32_t)(Smem::kA >> 4); b_lo += (uint32_t)(Smem::kB >> 4); }
+  }
+}
+
+// An epilogue warp's share of every tile: warp ew + 4 reads TMEM lane quarter q, i.e. tile rows q * 32 + lane.  Warp w may
+// only touch TMEM lanes 32*(w%4)..+31, so with EW = 8 two warps share each lane quarter and split the 32-column chunks
+// between them (chunk group cgrp); that doubles the epilogue throughput.
+struct EpiWarp {
+  int ew, q, cgrp;
+  int xl, yl, nl;      // this thread's row in the tile
+  int xl0, yl0, nl0;   // the quarter's first row: origin of its TMA-store sub-box
+  __device__ explicit EpiWarp(const TcConvParams& p) {
+    ew = (int)(threadIdx.x >> 5) - 4;
+    q = ew & 3;
+    cgrp = ew >> 2;
+    const int row = q * 32 + (threadIdx.x & 31), row0 = q * 32;
+    xl = row & (p.TW - 1);
+    yl = (row >> p.tw_log2) & (p.TH - 1);
+    nl = row >> (p.tw_log2 + p.th_log2);
+    xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
+  }
 };
 
-// EW = number of epilogue warps (4 or 8).  Warp w may only touch TMEM lanes 32*(w%4)..+31, so with
-// eight warps two warps share each lane quarter and split the 32-column chunks between them; that
-// doubles the epilogue throughput.
-template <int BN, int MT, int STAGES, int EW, bool INF>
-__global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const __grid_constant__ TcConvParams p, int n_ntiles,
-                                                                            int n_groups, int n_z, int n_work) {
-  static_assert(EW == 4 || EW == 8, "4 or 8 epilogue warps");
-  constexpr int kChunkGroups = EW / 4;
+// Epilogue warp, one 128-pixel tile at origin t: its lane quarter of the accumulator at TMEM address `acc` (zeros when the
+// item has no k-blocks), chunk by chunk through epilogue_chunk; pixels outside the grid, or all of them when !live, store
+// nothing.
+template <int BN, int EW, bool INF>
+__device__ __forceinline__ void drain_tile(const TcConvParams& p, const TcPhase& ph, const EpiWarp& e, uint32_t acc, bool has_k, Tile t,
+                                           bool live, int ncol0, int z, uint8_t* stage_base) {
+  const int gx = t.x0 + e.xl, gy = t.y0 + e.yl, gn = t.n0 + e.nl;
+  const bool valid = gx < p.gw && gy < p.gh && gn < p.gn && live;
+  const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
+#pragma unroll(EW == 4 ? BN / 32 : 1)
+  for (int i = 0; i < BN / EW / 8; ++i) {     // this warp's chunks
+    const int c = EW == 4 ? i : i * (EW / 4) + e.cgrp;
+    const int c0 = c * 32;
+    uint32_t r[32];
+    if (has_k) {
+      ptx::tmem_ld_32x32(acc + ((uint32_t)(e.q * 32) << 16) + (uint32_t)c0, r);
+      ptx::tmem_ld_wait();
+    } else {
+#pragma unroll
+      for (int j = 0; j < 32; ++j) r[j] = 0u;
+    }
+    epilogue_chunk<INF>(p, r, valid, opix, gn, ncol0 + c0, c == 0, stage_base + e.ew * kStageBytes, t.x0 + e.xl0, t.y0 + e.yl0,
+                        t.n0 + e.nl0, z);
+  }
+}
+
+// One-shot form: one CTA per (128-pixel tile, N tile, phase | k-split), two CTAs per SM.
+// warp 0 = TMA producer, warp 1 = MMA issuer, warp 2 = TMEM allocator, warps 4-7 = epilogue.
+template <int BN, int STAGES, bool INF>
+__global__ void __launch_bounds__(kTcThreads) tc_conv_kernel(const __grid_constant__ TcConvParams p) {
+  using Smem = ConvSmem<BN, STAGES>;
   extern __shared__ uint8_t smem_raw[];
-  constexpr int kBBytes = BN * 128;
-  constexpr int kAStage = MT * kABytes;
+  const Smem sm(smem_raw);
+  uint64_t* const tmem_full = sm.acc;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int z = (int)blockIdx.z;
+  int kb0, kb1;
+  const TcPhase& ph = conv_slice(p, z, kb0, kb1);
+  const bool has_k = kb1 > kb0;
+  const Tile t = tile_origin(p, (int)blockIdx.x);
+  const int ncol0 = blockIdx.y * BN;
+  const uint32_t tmem_base = tc_prologue<1, BN>(sm, &p.w_map, &p.in_maps[0], [&] { ptx::mbar_init(tmem_full, 1); });
+
+  if (has_k) {
+    RingPos<Smem> pos;
+    if (warp == 0) {
+      const Tile ts[1] = {t};
+      load_item<1, 1>(p, ph, kb0, kb1, ts, 1, ncol0, 0, sm, pos);
+    } else if (warp == 1) {
+      const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sm.a), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sm.b), 16);
+      uint32_t a_lo = a_lo0, b_lo = b_lo0;
+      mma_item<1, BN, 1>(tmem_base, kb1 - kb0, 1, sm, pos, a_lo0, b_lo0, a_lo, b_lo);
+      if (ptx::elect_one()) ptx::mma_commit(tmem_full);
+      __syncwarp();
+    }
+  }
+
+  if (warp >= 4) {
+    if (has_k) {
+      ptx::mbar_wait(tmem_full, 0);
+      ptx::tc_fence_after();
+    }
+    // deterministic split-K: this split's reductions go after those of split z - 1 of the same output tile
+    int* const det_lock = (p.det_locks != nullptr && p.ksplit > 1) ? p.det_locks + (blockIdx.y * gridDim.x + blockIdx.x) : nullptr;
+    if (det_lock) {
+      if (lane == 0) det_wait_turn(det_lock, z);
+      __syncwarp();
+    }
+    // an empty k-split adds nothing, but with per-split slabs it stores its zeros
+    const bool live = !(p.ksplit > 1 && !has_k && p.det_split_stride == 0);
+    drain_tile<BN, 4, INF>(p, ph, EpiWarp(p), tmem_base, has_k, t, live, ncol0, z, sm.stage);
+    if (det_lock) {
+      __threadfence();
+      asm volatile("bar.sync 2, 128;" ::: "memory");      // the four epilogue warps
+      if (warp == 4 && lane == 0) det_publish_turn(det_lock, z + 1 == p.ksplit ? 0 : z + 1);
+    }
+    if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
+  }
+  tc_teardown<1, BN>(tmem_base);
+}
+
+// Persistent forms: one CTA per SM (CTAS = 1, tc_conv_persist_kernel) or one CTA pair per two SMs (CTAS = 2,
+// tc_conv_pair_kernel) loops over work items (phase | k-split, N tile, group of CTAS x MT pixel tiles).  The TMEM accumulator
+// is double-buffered so the epilogue of item i overlaps the main loop of item i+1, and the MT pixel tiles of a CTA share
+// every staged weight tile.  Warps as in the one-shot form, with EW epilogue warps (4 or 8).
+//
+// CTA pairs (cta_group::2): the two CTAs of a cluster - two SMs - issue ONE M=256 MMA.  Each CTA stages its own MT pixel
+// tiles (A, 128 rows each) and HALF of the weight tile (B, BN/2 rows); the tensor core of each SM reads its own A and both
+// halves of B, so the per-SM shared-memory reads per MMA drop from (4 KB + BN*32 B) to (4 KB + BN*16 B) and the staged weight
+// bytes halve as well.  Protocol (leader = cluster rank 0):
+//   * producer warp in BOTH CTAs: waits its own empty[s] (multicast commit), issues its TMA loads with the completion bytes
+//     counted on the LEADER's full[s]; the leader arms full[s] with the bytes of both CTAs;
+//   * MMA warp in the leader only; tcgen05.commit multicasts to empty[s] / acc_full[a] of both CTAs;
+//   * epilogue warps in both CTAs drain their own TMEM and arrive (cluster scope) on the leader's acc_empty[a], which
+//     therefore counts 2*EW arrivals.
+// Requires total pixel tiles % (2*MT) == 0 (the host falls back to the single-CTA kernel otherwise).
+template <int CTAS, int BN, int MT, int STAGES, int EW, bool INF>
+__device__ __forceinline__ void conv_persistent(const TcConvParams& p, int n_ntiles, int n_groups, int n_work) {
+  static_assert(EW == 4 || EW == 8, "4 or 8 epilogue warps");
   constexpr int kAccCols = MT * BN;
   constexpr int kTmemCols = 2 * kAccCols;
   static_assert(kTmemCols <= 512 && kTmemCols >= 32, "TMEM budget");
-  const uint32_t raw_addr = ptx::smem_u32(smem_raw);
-  uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + STAGES * kAStage;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sB + STAGES * kBBytes);
-  uint64_t* empty = full + STAGES;
-  uint64_t* acc_full = empty + STAGES;       // [2]
-  uint64_t* acc_empty = acc_full + 2;        // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
-  // 512-byte aligned: the staging buffers' XOR pattern is then exactly TMA's 64-byte swizzle (absolute address bits)
-  uint8_t* stage_base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 511) & ~(uintptr_t)511);
-
+  using Smem = ConvPersistSmem<CTAS, BN, MT, STAGES, EW>;
+  extern __shared__ uint8_t smem_raw[];
+  const Smem sm(smem_raw);
+  uint64_t* const acc_full = sm.acc;        // [2]
+  uint64_t* const acc_empty = sm.acc + 2;   // [2]
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const uint32_t rank = CTAS == 2 ? ptx::cluster_ctarank() : 0u;
+  const int w_first = blockIdx.x / CTAS, w_step = gridDim.x / CTAS;
   const int total_tiles = p.tiles_x * p.tiles_y * p.tiles_n;
-
-  if (warp == 0 && lane == 0) {
-    ptx::prefetch_tmap(&p.w_map);
-    ptx::prefetch_tmap(&p.in_maps[0]);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
+  const uint32_t tmem_base = tc_prologue<CTAS, kTmemCols>(sm, &p.w_map, &p.in_maps[0], [&] {
     for (int a = 0; a < 2; ++a) {
       ptx::mbar_init(&acc_full[a], 1);
-      ptx::mbar_init(&acc_empty[a], EW);     // one arrival per epilogue warp
+      ptx::mbar_init(&acc_empty[a], CTAS * EW);     // one arrival per epilogue warp of the CTA (of both CTAs of a pair)
     }
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) ptx::tmem_alloc<kTmemCols>(tmem_slot);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  vg::pdl_entry();   // barriers, TMEM and descriptor prefetch above overlap the previous kernel's tail; nothing above touches global memory
-  const uint32_t tmem_base = *tmem_slot;
+  });
 
   // work item -> (z, n tile, pixel-tile group); groups vary fastest so that concurrently running
   // CTAs stream the same weight tile (L2 reuse) over neighbouring pixels
@@ -497,425 +620,107 @@ __global__ void __launch_bounds__(128 + 32 * EW, 1) tc_conv_persist_kernel(const
     nt = r / n_groups;
     g = r - nt * n_groups;
   };
-  auto k_range = [&](int z, const TcPhase& ph, int& kb0, int& kb1) {
-    const int total = ph.ntaps * p.k_chunks;
-    if (p.ksplit > 1) { kb0 = z * p.k_per_split; kb1 = min(total, kb0 + p.k_per_split); }
-    else { kb0 = 0; kb1 = total; }
-    if (kb1 < kb0) kb1 = kb0;
-  };
-  auto tile_origin = [&](int t, int& x0, int& y0, int& n0) {
-    t = min(t, total_tiles - 1);
-    const int tx = t % p.tiles_x; t /= p.tiles_x;
-    const int ty = t % p.tiles_y;
-    const int tn = t / p.tiles_y;
-    x0 = tx * p.TW; y0 = ty * p.TH; n0 = tn * p.TN;
-  };
-
-  // Producer and MMA warps run their loops WARP-UNIFORMLY and elect one lane only around the TMA / MMA
-  // issue (under a divergent `lane == 0` branch nvcc wraps every uniform-datapath instruction - UTMALDG,
-  // UTCHMMA, UTCBAR - in an elect-and-retry loop).
-  // One full/empty barrier pair per k-block: sharing one pair between two k-blocks halves the ~135-cycle
-  // wait bubbles of the MMA thread (NOTES above), but measured on B200 it brought nothing and cost the
-  // 256-wide tiles 8 % (coarser refill granularity; DESIGN.md 3.3 item 2), so that variant was removed.
-  if (warp == 0) {
-    int stage = 0;
-    uint32_t phase = 0;
-    for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-      int z, nt, g;
-      decode(w, z, nt, g);
-      const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-      int kb0, kb1;
-      k_range(z, ph, kb0, kb1);
-      if (kb1 == kb0) continue;
-      const int tile0 = g * MT;
-      const int nvalid = min(MT, total_tiles - tile0);
-      int x0s[MT], y0s[MT], n0s[MT];
-#pragma unroll
-      for (int m = 0; m < MT; ++m) tile_origin(tile0 + m, x0s[m], y0s[m], n0s[m]);
-      const int ncol0 = nt * BN;
-      int tp = kb0 / p.k_chunks, kc = kb0 % p.k_chunks;
-      for (int i = kb0; i < kb1; ++i) {
-        const TcTap tap = ph.taps[tp];
-        const CUtensorMap* im = &p.in_maps[tap.map];
-        ptx::mbar_wait(&empty[stage], phase ^ 1u);
-        if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(&full[stage], nvalid * kABytes + kBBytes);
-#pragma unroll
-          for (int m = 0; m < MT; ++m)
-            if (m < nvalid)
-              ptx::tma_load_4d(sA + stage * kAStage + m * kABytes, im, &full[stage], kc * 64, x0s[m] + tap.dx, y0s[m] + tap.dy, n0s[m]);
-          ptx::tma_load_2d(sB + stage * kBBytes, &p.w_map, &full[stage], kc * 64, tap.wrow + ncol0);
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-        if (++kc == p.k_chunks) { kc = 0; ++tp; }
-      }
-    }
-  } else if (warp == 1) {
-    constexpr uint32_t idesc = ptx::make_idesc_bf16(128, BN, 0, 0);
-    constexpr uint32_t kDescHi = ptx::smem_desc_hi(1024);
-    const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sA), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sB), 16);
-    uint32_t a_lo = a_lo0, b_lo = b_lo0;      // descriptor low words of the current stage
-    int stage = 0;
-    uint32_t phase = 0;
-    int it = 0;                       // number of accumulator uses so far
-    for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-      int z, nt, g;
-      decode(w, z, nt, g);
-      const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-      int kb0, kb1;
-      k_range(z, ph, kb0, kb1);
-      if (kb1 == kb0) continue;
-      const int nvalid = min(MT, total_tiles - g * MT);
-      const int as = it & 1;
-      ptx::mbar_wait(&acc_empty[as], (uint32_t)(((it >> 1) & 1) ^ 1));
-      ptx::tc_fence_after();
-      const uint32_t acc = tmem_base + (uint32_t)(as * kAccCols);
-      for (int i = kb0; i < kb1; ++i) {
-        ptx::mbar_wait(&full[stage], phase);
-        ptx::tc_fence_after();
-        if (ptx::elect_one()) {
-#pragma unroll
-          for (int m = 0; m < MT; ++m) {
-            if (m < nvalid) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                ptx::mma_bf16_ss_lohi(acc + (uint32_t)(m * BN), a_lo + (uint32_t)((m * kABytes + k * 32) >> 4),
-                                      b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc, (i > kb0) || (k > 0));
-            }
-          }
-          ptx::mma_commit(&empty[stage]);
-        }
-        __syncwarp();
-        if (++stage == STAGES) { stage = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
-        else { a_lo += (uint32_t)(kAStage >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
-      }
-      if (ptx::elect_one()) ptx::mma_commit(&acc_full[as]);
-      __syncwarp();
-      ++it;
-    }
-    vg::pdl_tail_trigger();
-  } else if (warp >= 4) {
-    const int ew = warp - 4;
-    const int q = ew & 3;                 // TMEM lane quarter this warp may access
-    const int cgrp = ew >> 2;             // which share of the 32-column chunks it handles
-    const int row = q * 32 + lane;
-    const int xl = row & (p.TW - 1);
-    const int yl = (row >> p.tw_log2) & (p.TH - 1);
-    const int nl = row >> (p.tw_log2 + p.th_log2);
-    // first pixel of this warp's 32-row quarter inside the tile: origin of its TMA-store sub-box
-    const int row0 = q * 32;
-    const int xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
-    int it = 0;
-    for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
-      int z, nt, g;
-      decode(w, z, nt, g);
-      const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-      int kb0, kb1;
-      k_range(z, ph, kb0, kb1);
-      const bool has_k = kb1 > kb0;
-      if (!has_k && p.ksplit > 1) continue;          // empty k-split: contributes nothing
-      const int tile0 = g * MT;
-      const int nvalid = min(MT, total_tiles - tile0);
-      const int ncol0 = nt * BN;
-      const int as = it & 1;
-      if (has_k) {
-        ptx::mbar_wait(&acc_full[as], (uint32_t)((it >> 1) & 1));
-        ptx::tc_fence_after();
-      }
-      const uint32_t acc = tmem_base + (uint32_t)(as * kAccCols) + ((uint32_t)(q * 32) << 16);
-#pragma unroll 1
-      for (int m = 0; m < nvalid; ++m) {
-        int x0, y0, n0;
-        tile_origin(tile0 + m, x0, y0, n0);
-        const int gx = x0 + xl, gy = y0 + yl, gn = n0 + nl;
-        const bool valid = gx < p.gw && gy < p.gh && gn < p.gn;
-        const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
-#pragma unroll
-        for (int c = 0; c < BN / 32; ++c) {
-          if ((c % kChunkGroups) != cgrp) continue;
-          const int c0 = c * 32;
-          uint32_t r[32];
-          if (has_k) {
-            ptx::tmem_ld_32x32(acc + (uint32_t)(m * BN + c0), r);
-            ptx::tmem_ld_wait();
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) r[j] = 0u;
-          }
-          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + ew * kStageBytes,
-                              x0 + xl0, y0 + yl0, n0 + nl0, z);
-        }
-      }
-      if (has_k) {
-        // this warp is done reading accumulator stage `as`: hand it back to the MMA warp
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(&acc_empty[as]);
-        ++it;
-      }
-    }
-    if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
-  }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 2) ptx::tmem_dealloc<kTmemCols>(tmem_base);
-}
-
-// ------------------------------------------------------------------------------------------
-// CTA-pair variant (cta_group::2): two CTAs of a cluster - two SMs - issue ONE M=256 MMA.  Each CTA
-// stages its own MT pixel tiles (A, 128 rows each) and HALF of the weight tile (B, BN/2 rows); the
-// tensor core of each SM reads its own A and both halves of B, so the per-SM shared-memory reads per
-// MMA drop from (4 KB + BN*32 B) to (4 KB + BN*16 B) and the staged weight bytes halve as well.
-// Protocol (leader = cluster rank 0):
-//   * producer thread in BOTH CTAs: waits its own empty[s] (multicast commit), issues its TMA loads
-//     with the completion bytes counted on the LEADER's full[s]; the leader arms full[s] with the
-//     bytes of both CTAs;
-//   * MMA thread in the leader only; tcgen05.commit multicasts to empty[s] / acc_full[a] of both CTAs;
-//   * epilogue warps in both CTAs drain their own TMEM and arrive (cluster scope) on the leader's
-//     acc_empty[a], which therefore counts 2*EW arrivals.
-// Requires total pixel tiles % (2*MT) == 0 (the host falls back to the single-CTA kernel otherwise).
-// ------------------------------------------------------------------------------------------
-template <int BN, int MT, int STAGES, int EW>
-struct ConvPairSmem {
-  static constexpr int kBBytes = (BN / 2) * 128;
-  static constexpr int kBytes = STAGES * (MT * kABytes + kBBytes) + (2 * STAGES + 4) * 8 + 16 + 1024 + EW * kStageBytes + 16 + 512;
-};
-
-template <int BN, int MT, int STAGES, int EW, bool INF>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
-    tc_conv_pair_kernel(const __grid_constant__ TcConvParams p, int n_ntiles, int n_groups, int n_z, int n_work) {
-  static_assert(EW == 4 || EW == 8, "4 or 8 epilogue warps");
-  constexpr int kChunkGroups = EW / 4;
-  extern __shared__ uint8_t smem_raw[];
-  constexpr int kBBytes = (BN / 2) * 128;
-  constexpr int kAStage = MT * kABytes;
-  constexpr int kAccCols = MT * BN;
-  constexpr int kTmemCols = 2 * kAccCols;
-  static_assert(kTmemCols <= 512 && kTmemCols >= 32, "TMEM budget");
-  const uint32_t raw_addr = ptx::smem_u32(smem_raw);
-  uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
-  uint8_t* sA = smem;
-  uint8_t* sB = smem + STAGES * kAStage;
-  uint64_t* full = reinterpret_cast<uint64_t*>(sB + STAGES * kBBytes);
-  uint64_t* empty = full + STAGES;
-  uint64_t* acc_full = empty + STAGES;       // [2]
-  uint64_t* acc_empty = acc_full + 2;        // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
-  // 512-byte aligned: the staging buffers' XOR pattern is then exactly TMA's 64-byte swizzle (absolute address bits)
-  uint8_t* stage_base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(tmem_slot + 4) + 511) & ~(uintptr_t)511);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = ptx::cluster_ctarank();
-  const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-  const int total_tiles = p.tiles_x * p.tiles_y * p.tiles_n;
-
-  if (warp == 0 && lane == 0) {
-    ptx::prefetch_tmap(&p.w_map);
-    ptx::prefetch_tmap(&p.in_maps[0]);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      ptx::mbar_init(&acc_full[a], 1);
-      ptx::mbar_init(&acc_empty[a], 2 * EW);   // every epilogue warp of both CTAs
-    }
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) ptx::tmem_alloc_pair<kTmemCols>(tmem_slot);
-  ptx::tc_fence_before();
-  ptx::cluster_sync();                         // barriers of BOTH CTAs exist before anyone signals them
-  ptx::tc_fence_after();
-  vg::pdl_entry();   // barriers, TMEM and descriptor prefetch above overlap the previous kernel's tail; nothing above touches global memory
-  const uint32_t tmem_base = *tmem_slot;
-
-  auto decode = [&](int w, int& z, int& nt, int& g) {
-    const int per_z = n_ntiles * n_groups;
-    z = w / per_z;
-    const int r = w - z * per_z;
-    nt = r / n_groups;
-    g = r - nt * n_groups;
-  };
-  auto k_range = [&](int z, const TcPhase& ph, int& kb0, int& kb1) {
-    const int total = ph.ntaps * p.k_chunks;
-    if (p.ksplit > 1) { kb0 = z * p.k_per_split; kb1 = min(total, kb0 + p.k_per_split); }
-    else { kb0 = 0; kb1 = total; }
-    if (kb1 < kb0) kb1 = kb0;
-  };
-  auto tile_origin = [&](int t, int& x0, int& y0, int& n0) {
-    const int tx = t % p.tiles_x; t /= p.tiles_x;
-    const int ty = t % p.tiles_y;
-    const int tn = t / p.tiles_y;
-    x0 = tx * p.TW; y0 = ty * p.TH; n0 = tn * p.TN;
+  // this CTA's first pixel tile of group g, and how many of its MT tiles exist (all of them in a pair)
+  auto tiles_of = [&](int g, int& tile0, int& nvalid) {
+    tile0 = (g * CTAS + (int)rank) * MT;
+    nvalid = CTAS == 2 ? MT : min(MT, total_tiles - tile0);
   };
 
   if (warp == 0) {
-    {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (int w = pair; w < n_work; w += n_pairs) {
-        int z, nt, g;
-        decode(w, z, nt, g);
-        const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-        int kb0, kb1;
-        k_range(z, ph, kb0, kb1);
-        if (kb1 == kb0) continue;
-        const int tile0 = (g * 2 + (int)rank) * MT;      // this CTA's pixel tiles of the pair's group
-        int x0s[MT], y0s[MT], n0s[MT];
+    RingPos<Smem> pos;
+    for (int w = w_first; w < n_work; w += w_step) {
+      int z, nt, g, kb0, kb1, tile0, nvalid;
+      decode(w, z, nt, g);
+      const TcPhase& ph = conv_slice(p, z, kb0, kb1);
+      if (kb1 == kb0) continue;
+      tiles_of(g, tile0, nvalid);
+      Tile t[MT];
 #pragma unroll
-        for (int m = 0; m < MT; ++m) tile_origin(tile0 + m, x0s[m], y0s[m], n0s[m]);
-        const int nrow0 = nt * BN + (int)rank * (BN / 2);  // this CTA's half of the weight tile
-        int tp = kb0 / p.k_chunks, kc = kb0 % p.k_chunks;
-        for (int i = kb0; i < kb1; ++i) {
-          const TcTap tap = ph.taps[tp];
-          const CUtensorMap* im = &p.in_maps[tap.map];
-          ptx::mbar_wait(&empty[stage], phase ^ 1u);
-          if (ptx::elect_one()) {
-            if (rank == 0) ptx::mbar_arrive_expect_tx(&full[stage], 2 * (kAStage + kBBytes));
-            const uint32_t bar = ptx::mapa(ptx::smem_u32(&full[stage]), 0);
-#pragma unroll
-            for (int m = 0; m < MT; ++m)
-              ptx::tma_load_4d_pair(sA + stage * kAStage + m * kABytes, im, bar, kc * 64, x0s[m] + tap.dx, y0s[m] + tap.dy, n0s[m]);
-            ptx::tma_load_2d_pair(sB + stage * kBBytes, &p.w_map, bar, kc * 64, tap.wrow + nrow0);
-          }
-          __syncwarp();
-          if (++stage == STAGES) { stage = 0; phase ^= 1u; }
-          if (++kc == p.k_chunks) { kc = 0; ++tp; }
-        }
-      }
+      for (int m = 0; m < MT; ++m) t[m] = tile_origin(p, tile0 + m);
+      load_item<CTAS, MT>(p, ph, kb0, kb1, t, nvalid, nt * BN + (int)rank * (BN / CTAS), rank, sm, pos);
     }
   } else if (warp == 1) {
     if (rank == 0) {
-      constexpr uint32_t idesc = ptx::make_idesc_bf16(256, BN, 0, 0);
-      constexpr uint32_t kDescHi = ptx::smem_desc_hi(1024);
-      const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sA), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sB), 16);
+      const uint32_t a_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sm.a), 16), b_lo0 = ptx::smem_desc_lo(ptx::smem_u32(sm.b), 16);
       uint32_t a_lo = a_lo0, b_lo = b_lo0;
-      int stage = 0;
-      uint32_t phase = 0;
-      int it = 0;
-      for (int w = pair; w < n_work; w += n_pairs) {
-        int z, nt, g;
+      RingPos<Smem> pos;
+      int it = 0;                       // number of accumulator uses so far
+      for (int w = w_first; w < n_work; w += w_step) {
+        int z, nt, g, kb0, kb1, tile0, nvalid;
         decode(w, z, nt, g);
-        const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-        int kb0, kb1;
-        k_range(z, ph, kb0, kb1);
+        conv_slice(p, z, kb0, kb1);
         if (kb1 == kb0) continue;
+        tiles_of(g, tile0, nvalid);
         const int as = it & 1;
         ptx::mbar_wait(&acc_empty[as], (uint32_t)(((it >> 1) & 1) ^ 1));
         ptx::tc_fence_after();
-        const uint32_t acc = tmem_base + (uint32_t)(as * kAccCols);
-        for (int i = kb0; i < kb1; ++i) {
-          ptx::mbar_wait(&full[stage], phase);
-          ptx::tc_fence_after();
-          if (ptx::elect_one()) {
-#pragma unroll
-            for (int m = 0; m < MT; ++m) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                ptx::mma_bf16_ss_pair_lohi(acc + (uint32_t)(m * BN), a_lo + (uint32_t)((m * kABytes + k * 32) >> 4),
-                                           b_lo + (uint32_t)((k * 32) >> 4), kDescHi, idesc, (i > kb0) || (k > 0));
-            }
-            ptx::mma_commit_pair(&empty[stage], 3);
-          }
-          __syncwarp();
-          if (++stage == STAGES) { stage = 0; phase ^= 1u; a_lo = a_lo0; b_lo = b_lo0; }
-          else { a_lo += (uint32_t)(kAStage >> 4); b_lo += (uint32_t)(kBBytes >> 4); }
-        }
-        if (ptx::elect_one()) ptx::mma_commit_pair(&acc_full[as], 3);
+        mma_item<CTAS, BN, MT>(tmem_base + (uint32_t)(as * kAccCols), kb1 - kb0, nvalid, sm, pos, a_lo0, b_lo0, a_lo, b_lo);
+        if (ptx::elect_one()) commit_to<CTAS>(&acc_full[as]);
         __syncwarp();
         ++it;
       }
     }
-    vg::pdl_tail_trigger();
   } else if (warp >= 4) {
-    const int ew = warp - 4;
-    const int q = ew & 3;
-    const int cgrp = ew >> 2;
-    const int row = q * 32 + lane;
-    const int xl = row & (p.TW - 1);
-    const int yl = (row >> p.tw_log2) & (p.TH - 1);
-    const int nl = row >> (p.tw_log2 + p.th_log2);
-    // first pixel of this warp's 32-row quarter inside the tile: origin of its TMA-store sub-box
-    const int row0 = q * 32;
-    const int xl0 = row0 & (p.TW - 1), yl0 = (row0 >> p.tw_log2) & (p.TH - 1), nl0 = row0 >> (p.tw_log2 + p.th_log2);
+    const EpiWarp e(p);
     int it = 0;
-    for (int w = pair; w < n_work; w += n_pairs) {
-      int z, nt, g;
+    for (int w = w_first; w < n_work; w += w_step) {
+      int z, nt, g, kb0, kb1, tile0, nvalid;
       decode(w, z, nt, g);
-      const TcPhase& ph = p.phases[p.ksplit > 1 ? 0 : z];
-      int kb0, kb1;
-      k_range(z, ph, kb0, kb1);
+      const TcPhase& ph = conv_slice(p, z, kb0, kb1);
       const bool has_k = kb1 > kb0;
-      if (!has_k && p.ksplit > 1) continue;
-      const int tile0 = (g * 2 + (int)rank) * MT;
-      const int ncol0 = nt * BN;
+      if (!has_k && p.ksplit > 1) continue;          // empty k-split: contributes nothing
+      tiles_of(g, tile0, nvalid);
       const int as = it & 1;
       if (has_k) {
         ptx::mbar_wait(&acc_full[as], (uint32_t)((it >> 1) & 1));
         ptx::tc_fence_after();
       }
-      const uint32_t acc = tmem_base + (uint32_t)(as * kAccCols) + ((uint32_t)(q * 32) << 16);
 #pragma unroll 1
-      for (int m = 0; m < MT; ++m) {
-        int x0, y0, n0;
-        tile_origin(tile0 + m, x0, y0, n0);
-        const int gx = x0 + xl, gy = y0 + yl, gn = n0 + nl;
-        const bool valid = gx < p.gw && gy < p.gh && gn < p.gn;
-        const long long opix = ((long long)gn * p.OH + (long long)gy * p.os + ph.oy_off) * p.OW + (long long)gx * p.os + ph.ox_off;
-#pragma unroll
-        for (int c = 0; c < BN / 32; ++c) {
-          if ((c % kChunkGroups) != cgrp) continue;
-          const int c0 = c * 32;
-          uint32_t r[32];
-          if (has_k) {
-            ptx::tmem_ld_32x32(acc + (uint32_t)(m * BN + c0), r);
-            ptx::tmem_ld_wait();
-          } else {
-#pragma unroll
-            for (int j = 0; j < 32; ++j) r[j] = 0u;
-          }
-          epilogue_chunk<INF>(p, r, valid, p.ksplit <= 1 || z == 0, opix, gn, ncol0 + c0, c == 0, stage_base + ew * kStageBytes,
-                              x0 + xl0, y0 + yl0, n0 + nl0, z);
-        }
-      }
+      for (int m = 0; m < nvalid; ++m)
+        drain_tile<BN, EW, INF>(p, ph, e, tmem_base + (uint32_t)(as * kAccCols + m * BN), has_k, tile_origin(p, tile0 + m), true, nt * BN,
+                                z, sm.stage);
       if (has_k) {
+        // this warp is done reading accumulator stage `as`: hand it back to the MMA warp (of the leader)
         ptx::tc_fence_before();
         __syncwarp();
-        if (lane == 0) ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&acc_empty[as]), 0));
+        if (lane == 0) {
+          if constexpr (CTAS == 2) ptx::mbar_arrive_cluster(ptx::mapa(ptx::smem_u32(&acc_empty[as]), 0));
+          else ptx::mbar_arrive(&acc_empty[as]);
+        }
         ++it;
       }
     }
     if (!INF && p.tma_store && lane == 0) ptx::bulk_wait_group0();      // this warp's bulk stores have landed
   }
-  // neither CTA may retire while the other can still signal its barriers or read its shared memory
-  ptx::tc_fence_before();
-  ptx::cluster_sync();
-  if (warp == 2) ptx::tmem_dealloc_pair<kTmemCols>(tmem_base);
+  tc_teardown<CTAS, kTmemCols>(tmem_base);
+}
+
+template <int BN, int MT, int STAGES, int EW, bool INF>
+__global__ void __launch_bounds__(128 + 32 * EW, 1)
+    tc_conv_persist_kernel(const __grid_constant__ TcConvParams p, int n_ntiles, int n_groups, int n_work) {
+  conv_persistent<1, BN, MT, STAGES, EW, INF>(p, n_ntiles, n_groups, n_work);
+}
+
+template <int BN, int MT, int STAGES, int EW, bool INF>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128 + 32 * EW, 1)
+    tc_conv_pair_kernel(const __grid_constant__ TcConvParams p, int n_ntiles, int n_groups, int n_work) {
+  conv_persistent<2, BN, MT, STAGES, EW, INF>(p, n_ntiles, n_groups, n_work);
 }
 
 // ------------------------------------------------------------------------------------------
 // weight gradient
 // ------------------------------------------------------------------------------------------
 template <int NB, int STAGES>
-struct WgradSmem {
-  static constexpr int kStageBytes = (2 + NB) * 8192;
-  static constexpr int kBytes = STAGES * kStageBytes + (2 * STAGES + 1) * 8 + 16 + 1024;
-};
-
-template <int NB, int STAGES>
 __global__ void __launch_bounds__(kTcThreads) tc_wgrad_kernel(const __grid_constant__ TcWgradParams p) {
+  using Smem = WgradSmem<NB, STAGES>;
   extern __shared__ uint8_t smem_raw[];
   constexpr int BN = NB * 64;
-  constexpr int kStageBytes = (2 + NB) * 8192;
-  const uint32_t raw_addr = ptx::smem_u32(smem_raw);
-  uint8_t* smem = smem_raw + ((1024u - (raw_addr & 1023u)) & 1023u);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + STAGES * kStageBytes);
-  uint64_t* empty = full + STAGES;
-  uint64_t* tmem_full = empty + STAGES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tmem_full + 1);
+  constexpr int kStageBytes = Smem::kA;
+  const Smem sm(smem_raw);
+  uint8_t* const smem = sm.a;
+  uint64_t* const full = sm.full;
+  uint64_t* const empty = sm.empty;
+  uint64_t* const tmem_full = sm.acc;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_slabs = p.ntaps * p.cs_chunks;
@@ -926,27 +731,10 @@ __global__ void __launch_bounds__(kTcThreads) tc_wgrad_kernel(const __grid_const
   const int box_end = min(p.n_boxes, box_begin + p.boxes_per_split);
   const int num_k = max(0, box_end - box_begin);
 
-  if (warp == 0 && lane == 0) {
-    ptx::prefetch_tmap(&p.u_map);
-    ptx::prefetch_tmap(&p.s_maps[0]);
-  }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) {
-      ptx::mbar_init(&full[s], 1);
-      ptx::mbar_init(&empty[s], 1);
-    }
-    ptx::mbar_init(tmem_full, 1);
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) ptx::tmem_alloc<(BN < 32 ? 32 : BN)>(tmem_slot);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  vg::pdl_entry();   // barriers, TMEM and descriptor prefetch above overlap the previous kernel's tail; nothing above touches global memory
-  const uint32_t tmem_base = *tmem_slot;
+  const uint32_t tmem_base = tc_prologue<1, BN>(sm, &p.u_map, &p.s_maps[0], [&] { ptx::mbar_init(tmem_full, 1); });
 
   if (num_k > 0) {
-    // role warps loop warp-uniformly; one elected lane issues the TMA / MMA instructions (see tc_conv_kernel)
+    // role warps loop warp-uniformly; one elected lane issues the TMA / MMA instructions (NOTES above)
     if (warp == 0) {
       const int tapA = slab0 / p.cs_chunks, chA = slab0 % p.cs_chunks;
       const int tapB = slab1 / p.cs_chunks, chB = slab1 % p.cs_chunks;
@@ -954,11 +742,8 @@ __global__ void __launch_bounds__(kTcThreads) tc_wgrad_kernel(const __grid_const
       int stage = 0;
       uint32_t phase = 0;
       for (int b = box_begin; b < box_end; ++b) {
-        int t = b;
-        const int tx = t % p.tiles_x; t /= p.tiles_x;
-        const int ty = t % p.tiles_y;
-        const int tn = t / p.tiles_y;
-        const int x0 = tx * p.TW, y0 = ty * p.TH, n0 = tn * p.TN;
+        const Tile t = tile_origin(p, b);
+        const int x0 = t.x0, y0 = t.y0, n0 = t.n0;
         ptx::mbar_wait(&empty[stage], phase ^ 1u);
         if (ptx::elect_one()) {
           ptx::mbar_arrive_expect_tx(&full[stage], kStageBytes);
@@ -995,7 +780,6 @@ __global__ void __launch_bounds__(kTcThreads) tc_wgrad_kernel(const __grid_const
       }
       if (ptx::elect_one()) ptx::mma_commit(tmem_full);
       __syncwarp();
-      vg::pdl_tail_trigger();
     }
   }
 
@@ -1051,9 +835,7 @@ __global__ void __launch_bounds__(kTcThreads) tc_wgrad_kernel(const __grid_const
     asm volatile("bar.sync 2, 128;" ::: "memory");        // the four epilogue warps
     if (warp == 4 && lane == 0) det_publish_turn(det_lock, blockIdx.z + 1 == gridDim.z ? 0 : (int)blockIdx.z + 1);
   }
-  ptx::tc_fence_before();
-  __syncthreads();
-  if (warp == 2) ptx::tmem_dealloc<(BN < 32 ? 32 : BN)>(tmem_base);
+  tc_teardown<1, BN>(tmem_base);
 }
 
 // dw[cu][cs][tap] += ws[tap][cs][cu]  (32x32 smem-tile transpose between cu and r = cs*taps+tap)
@@ -1110,75 +892,58 @@ static EncodeTiledFn get_encode() {
   return g_encode;
 }
 
+// cuTensorMapEncodeTiled of a bf16 tensor with `rank` dimensions (dims, byte strides and box innermost first); `what` names the
+// tensor in the error message
+static int encode_map(CUtensorMap* m, const char* what, int rank, const void* base, const cuuint64_t* dims, const cuuint64_t* strides,
+                      const cuuint32_t* box, CUtensorMapSwizzle swizzle, CUtensorMapL2promotion l2) {
+  EncodeTiledFn enc = get_encode();
+  if (!enc) {
+    set_error("cuTensorMapEncodeTiled entry point unavailable");
+    return VG_ECUDA;
+  }
+  bind_context_once();
+  const cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), dims, strides, box, estr,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle, l2, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) {
+    char shape[128];
+    int len = 0;
+    for (int i = 0; i < rank; ++i)
+      len += snprintf(shape + len, sizeof(shape) - len, " %llu/%u", (unsigned long long)dims[i], (unsigned)box[i]);
+    set_error("cuTensorMapEncodeTiled(%s) failed: %d (dim/box:%s)", what, (int)r, shape);
+    return VG_ECUDA;
+  }
+  return VG_OK;
+}
+
 // NHWC bf16 activation [n][h][w][c]; parity (py,px) with step `s` selects rows py, py+s, ... and
 // columns px, px+s, ...  Box = {64, TW, TH, TN}.
 static int make_act_map(CUtensorMap* m, const void* base, int n, int h, int w, int c, int s, int py, int px, int TW, int TH,
                         int TN) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    set_error("cuTensorMapEncodeTiled entry point unavailable");
-    return VG_ECUDA;
-  }
-  bind_context_once();
   const int hs = (h - py + s - 1) / s, ws = (w - px + s - 1) / s;
-  cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)std::max(ws, 1), (cuuint64_t)std::max(hs, 1), (cuuint64_t)n};
-  cuuint64_t strides[3] = {(cuuint64_t)s * c * 2, (cuuint64_t)s * w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)TN};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  void* addr = (void*)((const char*)base + ((size_t)py * w + px) * c * 2);
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, addr, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(activation) failed: %d (n=%d h=%d w=%d c=%d s=%d box=%d,%d,%d)", (int)r, n, h, w, c, s, TW, TH, TN);
-    return VG_ECUDA;
-  }
-  return VG_OK;
+  const cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)std::max(ws, 1), (cuuint64_t)std::max(hs, 1), (cuuint64_t)n};
+  const cuuint64_t strides[3] = {(cuuint64_t)s * c * 2, (cuuint64_t)s * w * c * 2, (cuuint64_t)h * w * c * 2};
+  const cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, (cuuint32_t)TN};
+  return encode_map(m, "activation", 4, (const char*)base + ((size_t)py * w + px) * c * 2, dims, strides, box,
+                    CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 // bf16 output tensor (N, OH, OW, C) as {32 channels, bx, by, bn} boxes with the 64-byte swizzle (TMA-store epilogue)
 // (s, py, px): the sub-grid of output pixels (py + s*i, px + s*j) a scatter phase writes (s = 1: the whole tensor)
-static int make_out_map(CUtensorMap* m, void* base, int n, int h, int w, int c, int bx, int by, int bn, int s = 1, int py = 0,
-                        int px = 0) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    set_error("cuTensorMapEncodeTiled entry point unavailable");
-    return VG_ECUDA;
-  }
-  bind_context_once();
+static int make_out_map(CUtensorMap* m, void* base, int n, int h, int w, int c, int bx, int by, int bn, int s, int py, int px) {
   const int hs = (h - py + s - 1) / s, ws = (w - px + s - 1) / s;
-  cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)std::max(ws, 1), (cuuint64_t)std::max(hs, 1), (cuuint64_t)n};
-  cuuint64_t strides[3] = {(cuuint64_t)s * c * 2, (cuuint64_t)s * w * c * 2, (cuuint64_t)h * w * c * 2};
-  cuuint32_t box[4] = {32, (cuuint32_t)bx, (cuuint32_t)by, (cuuint32_t)bn};
-  cuuint32_t estr[4] = {1, 1, 1, 1};
-  base = (void*)((char*)base + ((size_t)py * w + px) * c * 2);
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(output) failed: %d (n=%d h=%d w=%d c=%d box=%d,%d,%d)", (int)r, n, h, w, c, bx, by, bn);
-    return VG_ECUDA;
-  }
-  return VG_OK;
+  const cuuint64_t dims[4] = {(cuuint64_t)c, (cuuint64_t)std::max(ws, 1), (cuuint64_t)std::max(hs, 1), (cuuint64_t)n};
+  const cuuint64_t strides[3] = {(cuuint64_t)s * c * 2, (cuuint64_t)s * w * c * 2, (cuuint64_t)h * w * c * 2};
+  const cuuint32_t box[4] = {32, (cuuint32_t)bx, (cuuint32_t)by, (cuuint32_t)bn};
+  return encode_map(m, "output", 4, (char*)base + ((size_t)py * w + px) * c * 2, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_64B,
+                    CU_TENSOR_MAP_L2_PROMOTION_NONE);
 }
 
 static int make_weight_map(CUtensorMap* m, const void* base, long long rows, int k, int box_rows) {
-  EncodeTiledFn enc = get_encode();
-  if (!enc) {
-    set_error("cuTensorMapEncodeTiled entry point unavailable");
-    return VG_ECUDA;
-  }
-  bind_context_once();
-  cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)rows};
-  cuuint64_t strides[1] = {(cuuint64_t)k * 2};
-  cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-  cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) {
-    set_error("cuTensorMapEncodeTiled(weights) failed: %d (rows=%lld k=%d box_rows=%d)", (int)r, rows, k, box_rows);
-    return VG_ECUDA;
-  }
-  return VG_OK;
+  const cuuint64_t dims[2] = {(cuuint64_t)k, (cuuint64_t)rows};
+  const cuuint64_t strides[1] = {(cuuint64_t)k * 2};
+  const cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
+  return encode_map(m, "weights", 2, base, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 static int ilog2(int v) {
@@ -1202,103 +967,38 @@ static void choose_box(int gw, int gh, int gn, int pixels, int* TW, int* TH, int
   *TW = bw; *TH = bh; *TN = pixels / (bw * bh);
 }
 
-bool tc_conv_supported(const VgConvDesc* d, bool dgrad) {
+// what the forward / dgrad and the weight-gradient kernels both need: bf16 activations, stride 1 or 2, a square kernel of at
+// most 16 taps, even fine grids at stride 2 (parity maps / scatter phases), and the tensor-map encoder
+static bool tc_common_supported(const VgConvDesc* d) {
   if (g_force_simt) return false;
   if (d->act_dtype != VG_BF16) return false;
   if (d->stride != 1 && d->stride != 2) return false;
   if (d->kh != d->kw || d->kh * d->kw > 16) return false;
+  if (d->stride == 2 && ((d->transposed ? d->h_out : d->h_in) % 2 != 0 || (d->transposed ? d->w_out : d->w_in) % 2 != 0)) return false;
+  return get_encode() != nullptr;
+}
+
+bool tc_conv_supported(const VgConvDesc* d, bool dgrad) {
   const int c_red = dgrad ? d->c_out : d->c_in;
   const int n_out = dgrad ? d->c_in : d->c_out;
   // n_out == 1: the N tile is filled with the neighbouring taps' weight rows (finite garbage) and only
   // column 0 is stored - the reduction over 64+ input channels still runs on the tensor cores
-  if (c_red % 64 != 0 || (n_out % 64 != 0 && n_out != 1)) return false;
-  if (d->stride == 2 && ((d->transposed ? d->h_out : d->h_in) % 2 != 0 || (d->transposed ? d->w_out : d->w_in) % 2 != 0)) return false;
-  return get_encode() != nullptr;
+  return c_red % 64 == 0 && (n_out % 64 == 0 || n_out == 1) && tc_common_supported(d);
 }
 
 bool tc_wgrad_supported(const VgConvDesc* d) {
-  if (g_force_simt) return false;
-  if (d->act_dtype != VG_BF16) return false;
-  if (d->stride != 1 && d->stride != 2) return false;
-  if (d->kh != d->kw || d->kh * d->kw > 16) return false;
-  if (d->c_in % 64 != 0 || d->c_out % 64 != 0) return false;
-  if (d->stride == 2 && ((d->transposed ? d->h_out : d->h_in) % 2 != 0 || (d->transposed ? d->w_out : d->w_in) % 2 != 0)) return false;
-  return get_encode() != nullptr;
+  return d->c_in % 64 == 0 && d->c_out % 64 == 0 && tc_common_supported(d);
 }
 
-template <int BN, int STAGES, bool INF>
-static int launch_conv_t(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  static std::once_flag once;          // autograd worker threads call in concurrently
+// Launches one kernel instance with `smem` bytes of dynamic shared memory; the first launch of the instance raises its
+// shared-memory limit (once: autograd worker threads call in concurrently).
+template <auto Kernel, class... Args>
+static int launch(dim3 grid, int threads, int smem, cudaStream_t s, const Args&... args) {
+  static std::once_flag once;
   static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_kernel<BN, STAGES, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 ConvSmem<BN, STAGES>::kBytes); });
+  std::call_once(once, [smem] { attr_err = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); });
   VG_CUDA(attr_err);
-  vg::Launch(grid, kTcThreads, ConvSmem<BN, STAGES>::kBytes, s)(tc_conv_kernel<BN, STAGES, INF>, p);
-  VG_LAUNCHED();
-  return VG_OK;
-}
-
-template <int BN, int MT, int STAGES, int EW, bool INF>
-static int launch_conv_persist_t(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  static std::once_flag once;          // autograd worker threads call in concurrently
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_persist_kernel<BN, MT, STAGES, EW, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 ConvPersistSmem<BN, MT, STAGES, EW>::kBytes); });
-  VG_CUDA(attr_err);
-  const int n_groups = (int)cdiv(grid.x, MT);
-  const int n_ntiles = (int)grid.y;
-  const int n_z = (int)grid.z;
-  const long long n_work = (long long)n_groups * n_ntiles * n_z;
-  const int ctas = (int)std::min<long long>(n_work, num_sms());
-  vg::Launch(ctas, 128 + 32 * EW, ConvPersistSmem<BN, MT, STAGES, EW>::kBytes, s)(tc_conv_persist_kernel<BN, MT, STAGES, EW, INF>,
-      p, n_ntiles, n_groups, n_z, (int)n_work);
-  VG_LAUNCHED();
-  return VG_OK;
-}
-
-template <int BN, int MT, int STAGES, int EW, bool INF>
-static int launch_conv_pair_t(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  static std::once_flag once;          // autograd worker threads call in concurrently
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_conv_pair_kernel<BN, MT, STAGES, EW, INF>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 ConvPairSmem<BN, MT, STAGES, EW>::kBytes); });
-  VG_CUDA(attr_err);
-  const int n_groups = (int)(grid.x / (2 * MT));      // the caller checked divisibility
-  const int n_ntiles = (int)grid.y;
-  const int n_z = (int)grid.z;
-  const long long n_work = (long long)n_groups * n_ntiles * n_z;
-  const int pairs = (int)std::min<long long>(n_work, num_sms() / 2);
-  vg::Launch(2 * pairs, 128 + 32 * EW, ConvPairSmem<BN, MT, STAGES, EW>::kBytes, s)(tc_conv_pair_kernel<BN, MT, STAGES, EW, INF>, 
-      p, n_ntiles, n_groups, n_z, (int)n_work);
-  VG_LAUNCHED();
-  return VG_OK;
-}
-
-// the inference epilogue (activation / residual / second output) lives in its OWN instantiations: compiled into the
-// training kernels it cost them 12 % (b256 step 59.8 -> 67.3 ms: registers at the launch-bound cap, spills in the epilogue)
-template <int BN, int STAGES>
-static int launch_conv(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
-  return inf ? launch_conv_t<BN, STAGES, true>(p, grid, s) : launch_conv_t<BN, STAGES, false>(p, grid, s);
-}
-template <int BN, int MT, int STAGES, int EW>
-static int launch_conv_persist(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
-  return inf ? launch_conv_persist_t<BN, MT, STAGES, EW, true>(p, grid, s) : launch_conv_persist_t<BN, MT, STAGES, EW, false>(p, grid, s);
-}
-template <int BN, int MT, int STAGES, int EW>
-static int launch_conv_pair(const TcConvParams& p, dim3 grid, cudaStream_t s) {
-  const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
-  return inf ? launch_conv_pair_t<BN, MT, STAGES, EW, true>(p, grid, s) : launch_conv_pair_t<BN, MT, STAGES, EW, false>(p, grid, s);
-}
-
-template <int NB, int STAGES>
-static int launch_wgrad(const TcWgradParams& p, dim3 grid, cudaStream_t s) {
-  static std::once_flag once;          // autograd worker threads call in concurrently
-  static cudaError_t attr_err = cudaSuccess;
-  std::call_once(once, [] { attr_err = cudaFuncSetAttribute(tc_wgrad_kernel<NB, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, WgradSmem<NB, STAGES>::kBytes); });
-  VG_CUDA(attr_err);
-  vg::Launch(grid, kTcThreads, WgradSmem<NB, STAGES>::kBytes, s)(tc_wgrad_kernel<NB, STAGES>, p);
+  vg::Launch(grid, threads, smem, s)(Kernel, args...);
   VG_LAUNCHED();
   return VG_OK;
 }
@@ -1396,6 +1096,42 @@ static int pick_bn(int n_out) {
 // kernel-form heuristic of tc_conv_run (a tile-table form overrides it)
 constexpr int kPersistMinItemsPerSm64 = 6;   // 64-wide tiles go persistent from this many work items per SM on
 constexpr int kPairMinBN = 128;              // CTA pairs for 128- and 256-wide tiles; 64-wide tiles gain nothing (DESIGN.md 3.1)
+
+// persistent forms: (n_groups x N tiles x phases | k-splits) work items over at most one CTA per SM (CTAS = 2: one pair per
+// two SMs; the caller checked grid.x % (2 * MT) == 0)
+template <int CTAS, int BN, int MT, int STAGES, int EW, bool INF>
+static int launch_persistent(const TcConvParams& p, dim3 grid, cudaStream_t s) {
+  const int n_groups = (int)cdiv(grid.x, CTAS * MT);
+  const int n_work = (int)((long long)n_groups * grid.y * grid.z);
+  const int ctas = CTAS * std::min(n_work, num_sms() / CTAS);
+  const int threads = 128 + 32 * EW, smem = ConvPersistSmem<CTAS, BN, MT, STAGES, EW>::kBytes;
+  if constexpr (CTAS == 2)
+    return launch<tc_conv_pair_kernel<BN, MT, STAGES, EW, INF>>(ctas, threads, smem, s, p, (int)grid.y, n_groups, n_work);
+  else
+    return launch<tc_conv_persist_kernel<BN, MT, STAGES, EW, INF>>(ctas, threads, smem, s, p, (int)grid.y, n_groups, n_work);
+}
+
+// the kernel instance of each (form, N tile).  The inference epilogue (activation / residual / second output) lives in its
+// OWN instantiations (INF): compiled into the training kernels it cost them 12 % (b256 step 59.8 -> 67.3 ms: registers at
+// the launch-bound cap, spills in the epilogue).
+// 64-wide tiles are EPILOGUE-bound (9 k-blocks of N=64 MMAs per 128 x 64 outputs).  Eight epilogue warps instead of four
+// (<64,2,4,8>) measured NO gain on B200 (64->64 @96: 74.4 vs 74.9 us) and were removed: the bound was the store path
+// (32 lines per store instruction), addressed by the staged, coalesced stores of epilogue_chunk.
+template <bool INF>
+static int launch_conv(int form, int BN, const TcConvParams& p, dim3 grid, cudaStream_t s) {
+  switch (form * 1000 + BN) {
+    case kFormOneShot * 1000 + 64: return launch<tc_conv_kernel<64, 4, INF>>(grid, kTcThreads, ConvSmem<64, 4>::kBytes, s, p);
+    case kFormOneShot * 1000 + 128: return launch<tc_conv_kernel<128, 3, INF>>(grid, kTcThreads, ConvSmem<128, 3>::kBytes, s, p);
+    case kFormOneShot * 1000 + 256: return launch<tc_conv_kernel<256, 4, INF>>(grid, kTcThreads, ConvSmem<256, 4>::kBytes, s, p);
+    case kFormPersist * 1000 + 64: return launch_persistent<1, 64, 4, 3, 4, INF>(p, grid, s);
+    case kFormPersist * 1000 + 128: return launch_persistent<1, 128, 2, 4, 8, INF>(p, grid, s);
+    case kFormPersist * 1000 + 256: return launch_persistent<1, 256, 1, 4, 8, INF>(p, grid, s);
+    case kFormPair * 1000 + 64: return launch_persistent<2, 64, 4, 3, 4, INF>(p, grid, s);
+    case kFormPair * 1000 + 128: return launch_persistent<2, 128, 2, 4, 8, INF>(p, grid, s);
+    case kFormPair * 1000 + 256: return launch_persistent<2, 256, 1, 6, 8, INF>(p, grid, s);
+    default: set_error("unsupported BN %d", BN); return VG_EUNSUPPORTED;
+  }
+}
 
 // dgrad=false: y = conv(x).  dgrad=true: dx from dy.  `in` is the tensor being read.
 int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpack, const float* bias, const float* colscale,
@@ -1517,35 +1253,16 @@ int tc_conv_run(const VgConvDesc* d, bool dgrad, const void* in, const void* wpa
   const int form = p.ksplit > 1 ? kFormAuto : tuned.form;
   const bool use_persist = form == kFormAuto ? heur_persist : (form != kFormOneShot);
   // CTA pairs (cta_group::2) halve the per-SM shared-memory operand reads that bound the narrow tiles
+  int run_form = use_persist ? kFormPersist : kFormOneShot;
   if (use_persist && p.n_store != 1 && (form == kFormPair || (form == kFormAuto && BN >= kPairMinBN))) {
     const int mt = BN == 64 ? 4 : (BN == 128 ? 2 : 1);
     if (grid.x % (2 * mt) == 0) {
       if ((rc = make_weight_map(&p.w_map, wpack, (long long)k * k * n_out, in_c, BN / 2))) return rc;
-      switch (BN) {
-        case 64: return launch_conv_pair<64, 4, 3, 4>(p, grid, s);
-        case 128: return launch_conv_pair<128, 2, 4, 8>(p, grid, s);
-        case 256: return launch_conv_pair<256, 1, 6, 8>(p, grid, s);
-        default: break;
-      }
+      run_form = kFormPair;
     }
   }
-  // 64-wide tiles are EPILOGUE-bound (9 k-blocks of N=64 MMAs per 128 x 64 outputs).  Eight epilogue warps instead of four
-  // (<64,2,4,8>) measured NO gain on B200 (64->64 @96: 74.4 vs 74.9 us) and were removed: the bound was the store path
-  // (32 lines per store instruction), addressed by the staged, coalesced stores of epilogue_chunk.
-  if (use_persist) {
-    switch (BN) {
-      case 64: return launch_conv_persist<64, 4, 3, 4>(p, grid, s);
-      case 128: return launch_conv_persist<128, 2, 4, 8>(p, grid, s);
-      case 256: return launch_conv_persist<256, 1, 4, 8>(p, grid, s);
-      default: break;
-    }
-  }
-  switch (BN) {
-    case 64: rc = launch_conv<64, 4>(p, grid, s); break;
-    case 128: rc = launch_conv<128, 3>(p, grid, s); break;
-    case 256: rc = launch_conv<256, 4>(p, grid, s); break;
-    default: set_error("unsupported BN %d", BN); return VG_EUNSUPPORTED;
-  }
+  const bool inf = p.act_slope != 1.0f || p.residual != nullptr || p.out2 != nullptr;
+  rc = inf ? launch_conv<true>(run_form, BN, p, grid, s) : launch_conv<false>(run_form, BN, p, grid, s);
   if (rc == VG_OK && p.det_split_stride != 0)
     rc = ordered_reduce_f32((const float*)p.out, p.ksplit, p.det_split_stride, (float*)out, s);
   return rc;
@@ -1620,9 +1337,9 @@ int tc_wgrad_run(const VgConvDesc* d, const void* x, const void* dy, float* dw, 
     }
   }
   switch (NB) {
-    case 1: rc = launch_wgrad<1, 6>(p, grid, s); break;
-    case 2: rc = launch_wgrad<2, 5>(p, grid, s); break;
-    default: rc = launch_wgrad<4, 4>(p, grid, s); break;
+    case 1: rc = launch<tc_wgrad_kernel<1, 6>>(grid, kTcThreads, WgradSmem<1, 6>::kBytes, s, p); break;
+    case 2: rc = launch<tc_wgrad_kernel<2, 5>>(grid, kTcThreads, WgradSmem<2, 5>::kBytes, s, p); break;
+    default: rc = launch<tc_wgrad_kernel<4, 4>>(grid, kTcThreads, WgradSmem<4, 4>::kBytes, s, p); break;
   }
   if (rc == VG_OK && p.det_split_stride != 0) rc = ordered_reduce_f32(p.dw, (int)splits, p.det_split_stride, wgrad_dst, s);
   if (rc || !p.packed || acc_only) return rc;

@@ -84,24 +84,9 @@ static inline long long cdiv(long long a, long long b) { return (a + b - 1) / b;
 // previous kernel's - while the launch itself, the CTA rasterisation and whatever a kernel does BEFORE pdl_entry()
 // (mbarrier init, TMEM allocation, tensor-map prefetch in the tcgen05 / bulk-copy kernels) overlap the previous
 // kernel's tail.  Inside the captured iteration these become programmatic edges of the CUDA graph.
-// Measured on B200 (profiles/r2_pdl_ab.txt): batch 32 10.88 -> 10.59 ms/step, batch 256 unchanged.  An EARLY
-// `griddepcontrol.launch_dependents` right behind the wait (next grid resident while this one runs; build with
-// -DVG_PDL_TRIGGER=1) gave that gain back (10.88 ms) and cost 0.6 % at batch 256, so it is off.
-__device__ __forceinline__ void pdl_entry() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-#if defined(VG_PDL_TRIGGER) && VG_PDL_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-
-// experiment switch (-DVG_PDL_TAIL_TRIGGER=1): the long kernels signal `launch_dependents` when a CTA has issued its last
-// loads / MMAs, so the next grid's CTAs can take over SMs as this grid's CTAs retire instead of after the whole grid.
-// Measured on B200 (profiles/r2_pdl_ab.txt): 0.3 - 1.3 % SLOWER than the implicit trigger at CTA exit; off.
-__device__ __forceinline__ void pdl_tail_trigger() {
-#if defined(VG_PDL_TAIL_TRIGGER) && VG_PDL_TAIL_TRIGGER
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
+// Measured on B200 (profiles/r2_pdl_ab.txt): batch 32 10.88 -> 10.59 ms/step, batch 256 unchanged.  Kernels do not
+// trigger their dependents early (measured slower, DESIGN.md 3.5): the next grid starts once this one's CTAs have exited.
+__device__ __forceinline__ void pdl_entry() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 struct Launch {
   cudaLaunchConfig_t cfg;
